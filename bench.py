@@ -2,6 +2,7 @@
 """bench.py -- the measurement contract.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c1|c3|c2|mlp|c5]
+                    [--dump-outputs DIR]
 
 Default workload (``config.workload``): BASELINE.json configs[3], the C4 sweep at its largest size -- 2^20 independent
 pendulum trajectories x 200 save points, Float32 state / Float64 time -- per GPU (weak scaling: every rank integrates its
@@ -48,6 +49,7 @@ SENSE_DESC = ("ForwardDiffSensitivity (pendulum.jl:11): 1 primal + 2 dual-number
               "norm -- the library default (LDEQ_SENSE_FORWARD_DUAL) and what the reference arm computes")
 CPU_BUDGET_S = 150.0   # wall-clock bound of the CPU arm's timed steps
 TRAIN_GB, TRAIN_T = 65536, 50   # C5: global batch, frames per sequence
+DUMP_TRAJ_SAMPLE = 16384        # --dump-outputs: trajectories of the [T, B, z] result kept (the files stay under 64 MB)
 
 
 def workload_config(name, B, T):
@@ -274,6 +276,22 @@ def _bind_numa(local):
         return f"numa binding skipped: {type(e).__name__}"
 
 
+def dump_outputs(path, traj, dz0, dtheta, max_traj=DUMP_TRAJ_SAMPLE):
+    """`--dump-outputs DIR`: what a caller of the timed path receives from its last step, as .npy files, so that two
+    builds can be compared output for output on identical inputs.  traj.npy is the [T, n, z] trajectories
+    (ldeq_solve_fwd) of all B trajectories, or, when B > max_traj, of the fixed sample
+    sort(default_rng(0).choice(B, max_traj, replace=False)); dz0.npy [B, z] and dtheta.npy [B, p] are the whole gradient
+    (ldeq_solve_bwd).  At the C4 size that is 26 + 8 + 4 MB."""
+    import torch
+    B = traj.shape[1]
+    if B > max_traj:
+        idx = np.sort(np.random.default_rng(0).choice(B, max_traj, replace=False))
+        traj = traj[:, torch.from_numpy(idx).to(traj.device)]
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("traj", traj), ("dz0", dz0), ("dtheta", dtheta)):
+        np.save(os.path.join(path, f"{name}.npy"), a.cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -341,9 +359,12 @@ def run_ours(args):
             sampler.start()
         l0 = h.launch_count()
         evs = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(K)]
+        out = None
         barrier()
         for i in range(K):
-            step(evs[i])
+            out = step(evs[i])
+            if i < K - 1:
+                out = None   # only the last step's results are kept
         barrier()
         launches = h.launch_count() - l0
         clocks = sampler.stop() if sampler else None
@@ -351,16 +372,20 @@ def run_ours(args):
         bwd_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in evs]))
         # the step = the two kernel groups (the L2 flush of a small workload sits outside the event pairs)
         total_ms = allmax(float(np.sum([e[0].elapsed_time(e[2]) for e in evs])))
-        return {"ms_per_step": total_ms / K, "fwd_ms": fwd_ms, "bwd_ms": bwd_ms, "launches": int(launches), "clocks": clocks}
+        rec = {"ms_per_step": total_ms / K, "fwd_ms": fwd_ms, "bwd_ms": bwd_ms, "launches": int(launches), "clocks": clocks}
+        return rec, out
 
     # headline: the library default = the reference's own gradient (dual-number re-solves)
     opts_fd = ldeq.default_opts()
     assert opts_fd.sensealg == ldeq.SENSE_FORWARD_DUAL
-    fd = device_leg(opts_fd, K, W, sample_clocks=True)
+    fd, fd_out = device_leg(opts_fd, K, W, sample_clocks=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fd_out[0], *fd_out[1])
+    del fd_out
     value = world * B * (T - 1) / (fd["ms_per_step"] * 1e-3)
     # the explicit opt-in: discrete adjoint of the taped accepted steps
     opts_da = ldeq.default_opts(sensealg=ldeq.SENSE_DISCRETE_ADJOINT)
-    da = device_leg(opts_da, K, W)
+    da, _ = device_leg(opts_da, K, W)
 
     # ---- end to end through the host-buffer C-ABI entry points, ONE caller thread, pinned host memory -----------------
     hz0 = torch.from_numpy(z0n).pin_memory()
@@ -855,7 +880,11 @@ def main():
     ap.add_argument("--global-batch", type=int, default=65536, help="c5 only")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-training", action="store_true", help="skip the C5 training sub-record of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the trajectories and gradients of the last timed step as DIR/*.npy "
+                                                          "(GOKU workloads c1, c3, c4; rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in WORKLOADS):
+        ap.error(f"--dump-outputs needs --impl ours and a workload of {sorted(WORKLOADS)}")
     if args.workload in ("c2", "mlp"):
         if args.impl == "reference":
             run_latentode_reference(args)
