@@ -16,4 +16,7 @@ goku   ctypes front-end of ``libldeq_oracle.so`` (C++/OpenMP): per-trajectory Ts
 mlp    numpy restatement of the LatentODE matrix-state solve (``src/models/LatentODE.jl:61-78``)
        with its continuous and discrete adjoints.
 loss   numpy restatement of the ELBO reduction, reparameterised ``sample`` and Flux ``ADAMW``.
+recurrent  float64 torch loops of the recurrent pattern extractor.
+model  float64 torch restatement of whole GOKU_basic / LatentODE training steps over named parameters, with the
+       solve as an autograd node over ``goku`` / ``mlp``.
 """

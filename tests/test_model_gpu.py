@@ -75,12 +75,12 @@ def test_cpu_tensors_are_refused(ldeq):
         ldeq.goku_solve(torch.zeros(4, 2), torch.ones(4, 1), np.arange(5) * 0.05)
 
 
-def test_fused_recurrent_layers_equal_the_per_step_flux_loops(ldeq):
+def test_fused_recurrent_layers_equal_the_per_step_flux_loops(ldeq, monkeypatch):
     # the cuDNN route of the pattern extractor must be the same function (values and gradients) as the Flux-style loops
     from importlib import import_module
     model_mod = import_module("latentdiffeq_jl_b200.model")
     torch.manual_seed(3)
-    torch.backends.cudnn.allow_tf32 = False
+    monkeypatch.setattr(torch.backends.cudnn, "allow_tf32", False)   # restored when the test ends
     mt = ldeq.GOKU_basic()
     enc, dec = ldeq.default_layers(mt, 784, ldeq.Pendulum(), device=DEV)
     encoder = ldeq.Encoder(mt, enc)
@@ -90,12 +90,11 @@ def test_fused_recurrent_layers_equal_the_per_step_flux_loops(ldeq):
     x = torch.rand(30, 16, 784, device=DEV)
     outs = {}
     for fuse in (True, False):
-        model_mod.FUSE_RECURRENT = fuse
+        monkeypatch.setattr(model_mod, "FUSE_RECURRENT", fuse)
         encoder.zero_grad()
         mu, lv = encoder(x)
         (mu[0].square().sum() + mu[1].sum() + lv[0].sum() + lv[1].square().sum()).backward()
         outs[fuse] = ([m.detach().clone() for m in mu + lv], [p.grad.detach().clone() for p in encoder.parameters()])
-    model_mod.FUSE_RECURRENT = True
     for a, b in zip(outs[True][0], outs[False][0]):
         assert torch.allclose(a, b, rtol=1e-4, atol=1e-6)
     for a, b in zip(outs[True][1], outs[False][1]):
