@@ -29,6 +29,26 @@
  *     A solver failure of one trajectory is NOT an error: its (z,T) block is filled with NaN
  *     (GOKU.jl:114), retcode[b] says why, and its gradient contribution is zero.
  *   - One handle per GPU and host thread; a handle is not thread-safe.
+ *
+ * CUDA graph capture
+ *   Every entry point that takes a stream checks whether that stream is being captured (cudaStreamIsCapturing).  A
+ *   captured call records the same kernels and copies it would run eagerly; values the host passes are frozen into the
+ *   graph, so per-step values go through the _dev entry points below, which read them from device memory.
+ *   Capture-safe: ldeq_solve_fwd (no tape, or a FORWARD_DUAL tape) and ldeq_solve_bwd of such a tape, ldeq_tape_free,
+ *   ldeq_pattern_extractor_fwd / _bwd / ldeq_pe_tape_free, ldeq_sample / _dev, ldeq_elbo_* / _dev, ldeq_adamw_step /
+ *   _dev.  Rules:
+ *   - A tape recorded under capture has no host mirror and no event: its allocation and release become graph nodes.
+ *   - A captured solve reads an immutable device copy of its time grid, kept by the handle until ldeq_destroy (the grid
+ *     an eager call uses is overwritten when another grid arrives).  The copy is made by an eager solve on the same grid:
+ *     a capture whose grid has not been solved eagerly before is refused, since a copy from pageable host memory cannot
+ *     be captured.  Likewise the ELBO workspace, device scratch and the NVRTC variant of a user right-hand side for a
+ *     non-Tsit5 solver are created by a first eager call; under capture their absence is refused.
+ *   - Refused with LDEQ_ERR_UNSUPPORTED, before anything is enqueued (the capture stays valid and can be ended), because
+ *     they need the host while the work runs: a DISCRETE_ADJOINT tape and its reverse pass (the tape's overflow check,
+ *     tape_heal), ldeq_tape_overflow, ldeq_mlp_solve_fwd / _bwd and ldeq_mlp_bwd_stats (the MLP tape check and the
+ *     continuous adjoint), every _host entry point (staging and stream synchronisation), ldeq_allreduce_grads and
+ *     ldeq_allreduce_adamw_step (multi-GPU capture is not built).  ldeq_comm_unique_id / _init / _destroy take no stream:
+ *     they are set-up calls that synchronise the device and must not be made while a capture is open.
  */
 #ifndef LDEQ_H
 #define LDEQ_H
@@ -47,6 +67,14 @@ typedef struct ldeq_rhs ldeq_rhs;
 typedef struct ldeq_tape ldeq_tape;
 typedef struct ldeq_mlp_tape ldeq_mlp_tape;
 typedef void* ldeq_stream; /* cudaStream_t */
+
+/* Device-resident AdamW step state for ldeq_adamw_step_dev: the 1-based step count and the running Float64 products
+ * beta1^step, beta2^step that Flux keeps.  Zero-initialised step with beta1_pow = beta2_pow = 1 is the state before step 1. */
+typedef struct ldeq_adamw_state {
+    int64_t step;
+    double beta1_pow;
+    double beta2_pow;
+} ldeq_adamw_state;
 
 enum ldeq_status {
     LDEQ_OK = 0,
@@ -247,6 +275,11 @@ void ldeq_pe_tape_free(ldeq_handle* h, ldeq_pe_tape* tape, ldeq_stream stream);
 /* ---- reparameterised sample: z = mu + eps * exp(logvar/2), eps ~ N(0,1) drawn on the device ---- */
 int ldeq_sample(ldeq_handle* h, const float* mu, const float* logvar, float* z_out, float* eps_out /*opt*/,
                 int64_t n, uint64_t seed, uint64_t offset, ldeq_stream stream);
+/* The same with the offset taken from a device counter: increments *calls (device uint64) and draws at
+ * offset = *calls << 32, the value after the increment -- bit-identical to ldeq_sample at that offset.  For CUDA graphs:
+ * every replay draws new noise. */
+int ldeq_sample_dev(ldeq_handle* h, const float* mu, const float* logvar, float* z_out, float* eps_out /*opt*/,
+                    int64_t n, uint64_t seed, uint64_t* calls, ldeq_stream stream);
 
 /* ---- ELBO: L = sum_pixels mean_{B,T}(x-xhat)^2 + beta * sum_heads (1/B) sum 0.5(e^lv + mu^2 - lv - 1)
  * x, xhat (P,B,T); mu[h], logvar[h] (d_h,B) for n_heads heads (host arrays of device pointers).
@@ -263,6 +296,16 @@ int ldeq_elbo_logits_fwd_bwd(ldeq_handle* h, const float* x, const float* logits
                       const float* const* logvar_host, const int32_t* head_dims_host, int n_heads, float beta,
                       int B, int T, int P, float grad_scale, float* loss, float* dlogits, float* const* dmu_host,
                       float* const* dlogvar_host, ldeq_stream stream);
+/* Both with beta read from a device float (CUDA graphs: a replay uses the current value); results are bit-identical to
+ * the host-value calls with that beta. */
+int ldeq_elbo_fwd_bwd_dev(ldeq_handle* h, const float* x, const float* xhat, const float* const* mu_host,
+                          const float* const* logvar_host, const int32_t* head_dims_host, int n_heads, const float* beta,
+                          int B, int T, int P, float grad_scale, float* loss, float* dxhat, float* const* dmu_host,
+                          float* const* dlogvar_host, ldeq_stream stream);
+int ldeq_elbo_logits_fwd_bwd_dev(ldeq_handle* h, const float* x, const float* logits, const float* const* mu_host,
+                                 const float* const* logvar_host, const int32_t* head_dims_host, int n_heads, const float* beta,
+                                 int B, int T, int P, float grad_scale, float* loss, float* dlogits, float* const* dmu_host,
+                                 float* const* dlogvar_host, ldeq_stream stream);
 
 /* ---- fused multi-tensor AdamW with Flux semantics:
  * m = b1 m + (1-b1) g; v = b2 v + (1-b2) g^2; x -= lr * m/(1-b1^t) / (sqrt(v/(1-b2^t)) + eps) + decay * x
@@ -272,6 +315,12 @@ int ldeq_elbo_logits_fwd_bwd(ldeq_handle* h, const float* x, const float* logits
 int ldeq_adamw_step(ldeq_handle* h, float* params, const float* grads, float* m, float* v, int64_t n, double lr,
                     double beta1, double beta2, double eps, float decay, int64_t step, float grad_scale,
                     ldeq_stream stream);
+/* The same with the step taken from device memory: one single-thread kernel advances *state (step + 1, beta powers times
+ * beta1 / beta2, the multiplications of ldeq_adamw_step in the same order), then the update reads it.  Step k gives
+ * parameters, m and v bit-identical to ldeq_adamw_step(..., step = k).  For CUDA graphs: every replay is the next step. */
+int ldeq_adamw_step_dev(ldeq_handle* h, float* params, const float* grads, float* m, float* v, int64_t n, double lr,
+                        double beta1, double beta2, double eps, float decay, ldeq_adamw_state* state, float grad_scale,
+                        ldeq_stream stream);
 
 /* ---- gradient all-reduce FUSED with AdamW over NVLink peer memory (data-parallel training, model_train.jl:195-201
  * on several GPUs).  peer_grads_host[r] is rank r's flat gradient bucket mapped into this process (symmetric memory /

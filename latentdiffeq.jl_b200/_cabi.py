@@ -29,6 +29,7 @@ SYMBOLS = [
     "ldeq_mlp_solve_fwd", "ldeq_mlp_solve_bwd", "ldeq_mlp_tape_free", "ldeq_mlp_bwd_stats", "ldeq_debug_cadj_trace",
     "ldeq_pattern_extractor_param_count", "ldeq_pattern_extractor_fwd", "ldeq_pattern_extractor_bwd", "ldeq_pe_tape_free",
     "ldeq_sample", "ldeq_elbo_fwd_bwd", "ldeq_elbo_logits_fwd_bwd", "ldeq_adamw_step", "ldeq_allreduce_adamw_step",
+    "ldeq_sample_dev", "ldeq_elbo_fwd_bwd_dev", "ldeq_elbo_logits_fwd_bwd_dev", "ldeq_adamw_step_dev",
     "ldeq_comm_unique_id", "ldeq_comm_init", "ldeq_allreduce_grads", "ldeq_comm_destroy",
 ]
 COMM_ID_BYTES = 128
@@ -109,6 +110,10 @@ def load() -> C.CDLL:
     lib.ldeq_elbo_fwd_bwd.argtypes = [vp, vp, vp, vp, vp, vp, i32, flt, i32, i32, i32, flt, vp, vp, vp, vp, vp]
     lib.ldeq_elbo_logits_fwd_bwd.argtypes = lib.ldeq_elbo_fwd_bwd.argtypes
     lib.ldeq_adamw_step.argtypes = [vp, vp, vp, vp, vp, i64, dbl, dbl, dbl, dbl, flt, i64, flt, vp]
+    lib.ldeq_sample_dev.argtypes = [vp, vp, vp, vp, vp, i64, C.c_uint64, vp, vp]
+    lib.ldeq_elbo_fwd_bwd_dev.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp, i32, i32, i32, flt, vp, vp, vp, vp, vp]
+    lib.ldeq_elbo_logits_fwd_bwd_dev.argtypes = lib.ldeq_elbo_fwd_bwd_dev.argtypes
+    lib.ldeq_adamw_step_dev.argtypes = [vp, vp, vp, vp, vp, i64, dbl, dbl, dbl, dbl, flt, vp, flt, vp]
     lib.ldeq_allreduce_adamw_step.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp, i64, dbl, dbl, dbl, dbl, flt, i64, flt, vp]
     lib.ldeq_comm_unique_id.argtypes = [vp, vp]
     lib.ldeq_comm_init.argtypes = [vp, vp, i32, i32]

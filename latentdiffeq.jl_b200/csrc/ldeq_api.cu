@@ -30,6 +30,48 @@ int set_err(ldeq_handle* h, int code, const char* what, cudaError_t ce) {
     return code;
 }
 
+bool capturing(cudaStream_t s) {
+    cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+    return cudaStreamIsCapturing(s, &st) != cudaSuccess || st != cudaStreamCaptureStatusNone;
+}
+
+int refuse_capture(ldeq_handle* h, cudaStream_t s, const char* what, const char* why) {
+    if (!capturing(s)) return LDEQ_OK;
+    std::string msg = std::string(what) + ": not available under CUDA graph capture (" + why + ")";
+    return set_err(h, LDEQ_ERR_UNSUPPORTED, msg.c_str());
+}
+
+static bool same_grid(const std::vector<double>& a, const double* t, int T) {
+    return a.size() == (size_t)T && std::memcmp(a.data(), t, (size_t)T * sizeof(double)) == 0;
+}
+
+// An immutable device copy of the grid upload_tgrid has just put into d_tgrid (ldeq_handle::grid_cache).  Eager solves
+// never read these copies, so an unpinned one can be freed at any time.
+static int cache_grid(ldeq_handle* h, int T, cudaStream_t s) {
+    size_t lru = h->grid_cache.size();
+    int unpinned = 0;
+    for (size_t i = 0; i < h->grid_cache.size(); ++i) {
+        ldeq_handle::GridEntry& g = h->grid_cache[i];
+        if (same_grid(g.t, h->h_tgrid.data(), T)) { g.last_use = ++h->grid_clock; return LDEQ_OK; }
+        if (!g.pinned) {
+            ++unpinned;
+            if (lru == h->grid_cache.size() || g.last_use < h->grid_cache[lru].last_use) lru = i;
+        }
+    }
+    if (unpinned >= LDEQ_GRID_CACHE) {
+        LDEQ_CUDA(cudaFreeAsync(h->grid_cache[lru].d, s));
+        h->grid_cache.erase(h->grid_cache.begin() + lru);
+    }
+    ldeq_handle::GridEntry g;
+    LDEQ_CUDA(cudaMallocAsync((void**)&g.d, (size_t)T * sizeof(double), s));
+    LDEQ_CUDA(cudaMemcpyAsync(g.d, h->d_tgrid, (size_t)T * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    g.t = h->h_tgrid;
+    g.t0 = h->grid_t0; g.h = h->grid_h; g.uniform = h->grid_uniform;
+    g.last_use = ++h->grid_clock;
+    h->grid_cache.push_back(std::move(g));
+    return LDEQ_OK;
+}
+
 int upload_tgrid(ldeq_handle* h, const double* t_host, int T, cudaStream_t s) {
     if ((size_t)T > h->d_tgrid_cap) {
         // stream-ordered free so that kernels still reading the old grid finish first
@@ -41,7 +83,7 @@ int upload_tgrid(ldeq_handle* h, const double* t_host, int T, cudaStream_t s) {
         h->d_tgrid_cap = cap;
         h->h_tgrid.clear();
     }
-    if (h->h_tgrid.size() != (size_t)T || std::memcmp(h->h_tgrid.data(), t_host, (size_t)T * sizeof(double)) != 0) {
+    if (!same_grid(h->h_tgrid, t_host, T)) {
         h->h_tgrid.assign(t_host, t_host + T);
         h->grid_t0 = t_host[0];
         h->grid_h = T > 1 ? t_host[1] - t_host[0] : 0.0;
@@ -53,17 +95,29 @@ int upload_tgrid(ldeq_handle* h, const double* t_host, int T, cudaStream_t s) {
             if (std::fma((double)k, h->grid_h, h->grid_t0) != t_host[k]) h->grid_uniform = 0;
         // source is pageable host memory: the runtime stages it before returning
         LDEQ_CUDA(cudaMemcpyAsync(h->d_tgrid, t_host, (size_t)T * sizeof(double), cudaMemcpyHostToDevice, s));
+        return cache_grid(h, T, s);
     }
     return LDEQ_OK;
 }
 
-int ensure_scratch(ldeq_handle* h, int slot, size_t bytes) {
-    if (bytes <= h->scratch_cap[slot]) return LDEQ_OK;
+int ensure_scratch(ldeq_handle* h, int slot, size_t bytes, cudaStream_t s) {
+    const bool graph = capturing(s);
+    if (bytes <= h->scratch_cap[slot]) {
+        h->scratch_captured[slot] |= graph;
+        return LDEQ_OK;
+    }
+    if (graph) return set_err(h, LDEQ_ERR_UNSUPPORTED, "device scratch must grow, which cannot happen under CUDA graph capture: run the "
+                                                       "same call once outside the capture first");
     if (h->scratch[slot]) {
-        LDEQ_CUDA(cudaDeviceSynchronize());
-        LDEQ_CUDA(cudaFree(h->scratch[slot]));
+        if (h->scratch_captured[slot]) {
+            h->retired_scratch.push_back(h->scratch[slot]);  // a captured graph may still read it
+        } else {
+            LDEQ_CUDA(cudaDeviceSynchronize());
+            LDEQ_CUDA(cudaFree(h->scratch[slot]));
+        }
         h->scratch[slot] = nullptr;
         h->scratch_cap[slot] = 0;
+        h->scratch_captured[slot] = false;
     }
     size_t cap = bytes + bytes / 8 + 4096;
     cudaError_t e = cudaMalloc(&h->scratch[slot], cap);
@@ -183,6 +237,8 @@ static cudaError_t launch_user_fwdsens(void* const* fn, const ldeq_tape* tape, c
 // Pinned two-int mirrors + events come from a per-handle pool: cudaMallocHost / cudaFreeHost cost milliseconds of host time
 // (and the free synchronises the device), far more than a small solve.
 bool slot_acquire(ldeq_handle* h, int32_t** h_info, cudaEvent_t* ev) {
+    for (const ldeq_handle::Slot& sl : h->deferred_slots) slot_release(h, sl.h_info, sl.ev);
+    h->deferred_slots.clear();
     if (h->free_slots.empty()) {
         const int n = 64;
         int32_t* blk = nullptr;
@@ -207,8 +263,12 @@ void slot_release(ldeq_handle* h, int32_t* h_info, cudaEvent_t ev) {
     }
 }
 static bool slot_get(ldeq_handle* h, ldeq_tape* tape) { return slot_acquire(h, &tape->h_info, &tape->ready); }
-static void slot_put(ldeq_handle* h, ldeq_tape* tape) {
-    slot_release(h, tape->h_info, tape->ready);
+// Under capture the wait for the slot's copy is not allowed: the slot is handed back by the next slot_acquire instead.
+static void slot_put(ldeq_handle* h, ldeq_tape* tape, cudaStream_t s) {
+    if (tape->ready && capturing(s))
+        h->deferred_slots.push_back({tape->h_info, tape->ready});
+    else
+        slot_release(h, tape->h_info, tape->ready);
     tape->h_info = nullptr;
     tape->ready = nullptr;
 }
@@ -355,7 +415,10 @@ void ldeq_destroy(ldeq_handle* h) {
         for (int i = 0; i < LDEQ_MAX_SLABS; ++i) { cudaEventDestroy(h->ev_fwd[i]); cudaEventDestroy(h->ev_up[i]); }
         cudaEventDestroy(h->ev_join);
     }
+    for (auto& g : h->grid_cache) cudaFree(g.d);
+    for (void* p : h->retired_scratch) cudaFree(p);
     for (auto& sl : h->free_slots) cudaEventDestroy(sl.ev);
+    for (auto& sl : h->deferred_slots) cudaEventDestroy(sl.ev);
     for (auto* blk : h->pinned_blocks) cudaFreeHost(blk);
     delete h;
 }
@@ -386,12 +449,21 @@ int ldeq_rhs_dims(const ldeq_rhs* rhs, int* z_dim, int* p_dim) {
 
 namespace ldeq {
 
+// The device grid a solve reads: d_tgrid for eager calls, an immutable cache entry under capture.
+struct GridRef {
+    const double* d;
+    double t0, h;
+    int uniform;
+};
+static GridRef eager_grid(const ldeq_handle* h) { return GridRef{h->d_tgrid, h->grid_t0, h->grid_h, h->grid_uniform}; }
+
 // ---- one column slab of a solve -----------------------------------------------------------------------
 // All pointers are already offset to the slab's first trajectory; `ld` is the row stride of traj (trajectories of
-// the whole batch).  The grid has been uploaded (upload_tgrid) by the caller.
+// the whole batch).  The grid is on the device (upload_tgrid or the grid cache).  `graph`: the stream is capturing, so
+// a tape gets no host mirror of its statistics and no event.
 static int solve_fwd_slab(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const void* z0, const void* theta, const double* t_host,
-                          int B, int ld, int T, const ldeq_opts* opts, void* traj_out, int32_t* retcode, int32_t* naccept,
-                          int32_t* nreject, ldeq_tape** tape_out, cudaStream_t s) {
+                          const GridRef& grid, bool graph, int B, int ld, int T, const ldeq_opts* opts, void* traj_out,
+                          int32_t* retcode, int32_t* naccept, int32_t* nreject, ldeq_tape** tape_out, cudaStream_t s) {
     KOpts ko = to_kopts(opts);
     const int ZD = rhs->z_dim, PD = rhs->p_dim;
     const bool fwd_dual = tape_out && opts->sensealg == LDEQ_SENSE_FORWARD_DUAL;
@@ -402,7 +474,7 @@ static int solve_fwd_slab(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const 
         tape = new ldeq_tape();
         tape->dtype = dtype; tape->rhs_kind = rhs->kind; tape->rhs = rhs; tape->B = B; tape->T = T;
         tape->z_dim = ZD; tape->p_dim = PD; tape->kopts = ko;
-        tape->grid_t0 = h->grid_t0; tape->grid_h = h->grid_h; tape->grid_uniform = h->grid_uniform;
+        tape->grid_t0 = grid.t0; tape->grid_h = grid.h; tape->grid_uniform = grid.uniform;
         long long cap = opts->tape_steps;
         tape->sense = opts->sensealg;
         tape->solver = opts->solver;
@@ -421,24 +493,31 @@ static int solve_fwd_slab(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const 
         if (cap < 1) cap = 1;
         rc = tape_alloc(h, tape, (int)cap, s);
         if (rc) { delete tape; return rc; }
-        if (!slot_get(h, tape)) {
+        if (!graph && !slot_get(h, tape)) {
             cudaFreeAsync(tape->base, s);
             delete tape;
             return set_err(h, LDEQ_ERR_NOMEM, "tape host mirror");
         }
         // theta, the grid, the statistics and u0 (record 0) reach the tape through the forward kernel itself (TapeView)
     }
-    cudaError_t e = dispatch_fwd(h, opts->solver, rhs, dtype, z0, theta, h->d_tgrid, B, T, ko, traj_out, retcode, naccept, nreject, tape,
-                                 GridInfo{h->grid_t0, h->grid_h, h->grid_uniform, ld}, s);
+    cudaError_t e = dispatch_fwd(h, opts->solver, rhs, dtype, z0, theta, grid.d, B, T, ko, traj_out, retcode, naccept, nreject, tape,
+                                 GridInfo{grid.t0, grid.h, grid.uniform, ld}, s);
     h->launches += 1;
     if (e != cudaSuccess) {
-        if (tape) { cudaFreeAsync(tape->base, s); cudaEventRecord(tape->ready, s); slot_put(h, tape); delete tape; }
+        if (tape) {
+            cudaFreeAsync(tape->base, s);
+            if (tape->ready) cudaEventRecord(tape->ready, s);
+            slot_put(h, tape, s);
+            delete tape;
+        }
         if (rhs->kind < 0 && e == cudaErrorLaunchFailure && !h->err.empty() && h->err.compare(0, 5, "NVRTC") == 0) return LDEQ_ERR_COMPILE;
         return set_err(h, LDEQ_ERR_CUDA, "tsit5_fwd_kernel launch", e);
     }
     if (tape) {
-        cudaMemcpyAsync(tape->h_info, tape->info, 8, cudaMemcpyDeviceToHost, s);
-        cudaEventRecord(tape->ready, s);
+        if (tape->ready) {
+            cudaMemcpyAsync(tape->h_info, tape->info, 8, cudaMemcpyDeviceToHost, s);
+            cudaEventRecord(tape->ready, s);
+        }
         *tape_out = tape;
     }
     return LDEQ_OK;
@@ -492,7 +571,7 @@ static int check_solve_args(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, cons
 static void free_parts(ldeq_handle* h, ldeq_tape* tape, cudaStream_t s) {
     for (ldeq_tape* p : tape->parts) {
         if (p->base) cudaFreeAsync(p->base, s);
-        slot_put(h, p);
+        slot_put(h, p, s);
         delete p;
     }
     tape->parts.clear();
@@ -531,9 +610,9 @@ struct HostBufs {
     char *z0, *th, *traj, *dtraj, *dz0, *dth;
     int32_t *ret, *na, *nr;
 };
-static int host_bufs(ldeq_handle* h, size_t nz, size_t np, size_t nt, int B, bool fwd, bool bwd, HostBufs* hb) {
+static int host_bufs(ldeq_handle* h, size_t nz, size_t np, size_t nt, int B, bool fwd, bool bwd, HostBufs* hb, cudaStream_t s) {
     int rc;
-    if ((rc = ensure_scratch(h, 0, 2 * align_up(nz) + 2 * align_up(np) + 3 * align_up((size_t)B * 4)))) return rc;
+    if ((rc = ensure_scratch(h, 0, 2 * align_up(nz) + 2 * align_up(np) + 3 * align_up((size_t)B * 4), s))) return rc;
     char* in = (char*)h->scratch[0];
     hb->z0 = in; in += align_up(nz);
     hb->th = in; in += align_up(np);
@@ -543,8 +622,8 @@ static int host_bufs(ldeq_handle* h, size_t nz, size_t np, size_t nt, int B, boo
     hb->na = (int32_t*)in; in += align_up((size_t)B * 4);
     hb->nr = (int32_t*)in;
     hb->traj = hb->dtraj = nullptr;
-    if (fwd) { if ((rc = ensure_scratch(h, 1, nt))) return rc; hb->traj = (char*)h->scratch[1]; }
-    if (bwd) { if ((rc = ensure_scratch(h, 2, nt))) return rc; hb->dtraj = (char*)h->scratch[2]; }
+    if (fwd) { if ((rc = ensure_scratch(h, 1, nt, s))) return rc; hb->traj = (char*)h->scratch[1]; }
+    if (bwd) { if ((rc = ensure_scratch(h, 2, nt, s))) return rc; hb->dtraj = (char*)h->scratch[2]; }
     return LDEQ_OK;
 }
 
@@ -565,8 +644,27 @@ int ldeq_solve_fwd(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const void* z
     cudaStream_t s = (cudaStream_t)stream;
     LDEQ_CUDA(cudaSetDevice(h->device));
     if (B == 0) return LDEQ_OK;
-    if ((rc = upload_tgrid(h, t_host, T, s))) return rc;
-    return solve_fwd_slab(h, rhs, dtype, z0, theta, t_host, B, B, T, opts, traj_out, retcode, naccept, nreject, tape_out, s);
+    if (!capturing(s)) {
+        if ((rc = upload_tgrid(h, t_host, T, s))) return rc;
+        return solve_fwd_slab(h, rhs, dtype, z0, theta, t_host, eager_grid(h), false, B, B, T, opts, traj_out, retcode, naccept, nreject,
+                              tape_out, s);
+    }
+    // Under capture nothing may be enqueued before every check has passed, so that a refusal leaves the capture intact.
+    if (tape_out && opts->sensealg != LDEQ_SENSE_FORWARD_DUAL)
+        return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_fwd: a discrete-adjoint tape is not available under CUDA graph capture (its "
+                                                "reverse pass reads the tape's overflow count on the host)");
+    if (rhs->kind < 0 && opts->solver != LDEQ_SOLVER_TSIT5 && !rhs->alt[opts->solver].module)
+        return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_fwd: the right-hand side has not been compiled for this solver yet, and NVRTC "
+                                                "cannot run under CUDA graph capture: solve once outside the capture first");
+    ldeq_handle::GridEntry* g = nullptr;
+    for (auto& e : h->grid_cache)
+        if (same_grid(e.t, t_host, T)) { g = &e; break; }
+    if (!g)
+        return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_fwd: the time grid is not on the device, and a copy from host memory cannot be "
+                                                "captured: solve once on this grid outside the capture first");
+    g->pinned = true;  // the graph reads g->d for as long as the handle lives
+    return solve_fwd_slab(h, rhs, dtype, z0, theta, t_host, GridRef{g->d, g->t0, g->h, g->uniform}, true, B, B, T, opts, traj_out, retcode,
+                          naccept, nreject, tape_out, s);
 }
 
 int ldeq_solve_bwd(ldeq_handle* h, ldeq_tape* tape, const void* dtraj, void* dz0, void* dtheta, ldeq_stream stream) {
@@ -574,6 +672,14 @@ int ldeq_solve_bwd(ldeq_handle* h, ldeq_tape* tape, const void* dtraj, void* dz0
     if (!tape || !dtraj || !dz0 || !dtheta) return set_err(h, LDEQ_ERR_INVALID, "null argument");
     cudaStream_t s = (cudaStream_t)stream;
     LDEQ_CUDA(cudaSetDevice(h->device));
+    if (capturing(s)) {
+        if (!tape->parts.empty() || tape->sense != LDEQ_SENSE_FORWARD_DUAL)
+            return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_bwd: only the forward-dual pullback of a device solve is available under CUDA "
+                                                    "graph capture (the discrete adjoint reads the tape's overflow count on the host)");
+        if (tape->rhs_kind < 0 && tape->solver != LDEQ_SOLVER_TSIT5 && !tape->rhs->alt[tape->solver].module)
+            return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_bwd: the right-hand side has not been compiled for this solver yet, and "
+                                                    "NVRTC cannot run under CUDA graph capture");
+    }
     if (tape->parts.empty()) return solve_bwd_slab(h, tape, dtraj, tape->B, dz0, dtheta, s);
     // a tape recorded slab by slab (ldeq_solve_fwd_host): same column slabs of the device arrays
     const size_t es = tape->dtype == LDEQ_F32 ? 4 : 8;
@@ -587,10 +693,13 @@ int ldeq_solve_bwd(ldeq_handle* h, ldeq_tape* tape, const void* dtraj, void* dz0
     return LDEQ_OK;
 }
 
-int ldeq_tape_overflow(ldeq_handle* h, ldeq_tape* tape, int32_t* count_host, ldeq_stream) {
+int ldeq_tape_overflow(ldeq_handle* h, ldeq_tape* tape, int32_t* count_host, ldeq_stream stream) {
     if (!h || !tape || !count_host) return LDEQ_ERR_INVALID;
+    int rc = refuse_capture(h, (cudaStream_t)stream, "ldeq_tape_overflow", "it waits for the forward kernel and reads its result on the host");
+    if (rc) return rc;
     *count_host = 0;
     auto one = [&](ldeq_tape* t) -> int {
+        if (!t->ready) return LDEQ_OK;  // recorded under capture: a forward-dual tape, which cannot overflow
         LDEQ_CUDA(cudaEventSynchronize(t->ready));
         if (t->sense == LDEQ_SENSE_FORWARD_DUAL) return LDEQ_OK;  // the dual re-solves keep no step records: nothing can overflow
         *count_host += t->checked && t->h_info[0] > 0 && t->cap >= t->h_info[1] ? 0 : t->h_info[0];
@@ -606,7 +715,7 @@ void ldeq_tape_free(ldeq_handle* h, ldeq_tape* tape, ldeq_stream stream) {
     if (h) cudaSetDevice(h->device);
     free_parts(h, tape, (cudaStream_t)stream);
     if (tape->base) cudaFreeAsync(tape->base, (cudaStream_t)stream);
-    slot_put(h, tape);
+    slot_put(h, tape, (cudaStream_t)stream);
     delete tape;
 }
 
@@ -621,12 +730,13 @@ int ldeq_solve_fwd_host(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const vo
     if (!traj_out_host) return set_err(h, LDEQ_ERR_INVALID, "null argument");
     if (B <= 0) return set_err(h, LDEQ_ERR_INVALID, "B must be > 0");
     cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = refuse_capture(h, s, "ldeq_solve_fwd_host", "it stages through host memory and synchronises the stream"))) return rc;
     LDEQ_CUDA(cudaSetDevice(h->device));
     if ((rc = host_streams(h))) return rc;
     const size_t es = dtype == LDEQ_F32 ? 4 : 8, zb = (size_t)rhs->z_dim * es, pb = (size_t)rhs->p_dim * es;
     const size_t nz = (size_t)B * zb, np = (size_t)B * pb, nt = nz * (size_t)T;
     HostBufs hb;
-    if ((rc = host_bufs(h, nz, np, nt, B, true, false, &hb))) return rc;
+    if ((rc = host_bufs(h, nz, np, nt, B, true, false, &hb, s))) return rc;
     if ((rc = upload_tgrid(h, t_host, T, s))) return rc;
     LDEQ_CUDA(cudaMemcpyAsync(hb.z0, z0_host, nz, cudaMemcpyHostToDevice, s));
     LDEQ_CUDA(cudaMemcpyAsync(hb.th, theta_host, np, cudaMemcpyHostToDevice, s));
@@ -642,7 +752,7 @@ int ldeq_solve_fwd_host(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const vo
         slab_bounds(B, ns, i, &b0, &nb);
         if (nb <= 0) continue;
         ldeq_tape* part = nullptr;
-        rc = solve_fwd_slab(h, rhs, dtype, hb.z0 + b0 * zb, hb.th + b0 * pb, t_host, nb, B, T, opts, hb.traj + b0 * zb, hb.ret + b0,
+        rc = solve_fwd_slab(h, rhs, dtype, hb.z0 + b0 * zb, hb.th + b0 * pb, t_host, eager_grid(h), false, nb, B, T, opts, hb.traj + b0 * zb, hb.ret + b0,
                             hb.na + b0, hb.nr + b0, parent ? &part : nullptr, s);
         if (rc) { if (parent) { free_parts(h, parent, s); delete parent; } return rc; }
         if (parent) { parent->parts.push_back(part); parent->part_b0.push_back(b0); }
@@ -666,14 +776,15 @@ int ldeq_solve_bwd_host(ldeq_handle* h, ldeq_tape* tape, const void* dtraj_host,
     if (!h) return LDEQ_ERR_INVALID;
     if (!tape || !dtraj_host || !dz0_host || !dtheta_host) return set_err(h, LDEQ_ERR_INVALID, "null argument");
     cudaStream_t s = (cudaStream_t)stream;
-    LDEQ_CUDA(cudaSetDevice(h->device));
     int rc;
+    if ((rc = refuse_capture(h, s, "ldeq_solve_bwd_host", "it stages through host memory and synchronises the stream"))) return rc;
+    LDEQ_CUDA(cudaSetDevice(h->device));
     if ((rc = host_streams(h))) return rc;
     const size_t es = tape->dtype == LDEQ_F32 ? 4 : 8, zb = (size_t)tape->z_dim * es, pb = (size_t)tape->p_dim * es;
     const int B = tape->B, T = tape->T;
     const size_t nz = (size_t)B * zb, np = (size_t)B * pb, nt = nz * (size_t)T;
     HostBufs hb;
-    if ((rc = host_bufs(h, nz, np, nt, B, false, true, &hb))) return rc;
+    if ((rc = host_bufs(h, nz, np, nt, B, false, true, &hb, s))) return rc;
     // every part's cotangent slab goes up on the copy stream; its reverse pass follows on the caller's stream
     const size_t nparts = tape->parts.empty() ? 1 : tape->parts.size();
     LDEQ_CUDA(cudaEventRecord(h->ev_join, s));   // uploads must not overtake earlier work of the caller on this scratch
@@ -704,12 +815,13 @@ int ldeq_solve_fwd_bwd_host(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, cons
     if (!dtraj_host || !traj_out_host || !dz0_host || !dtheta_host) return set_err(h, LDEQ_ERR_INVALID, "null argument");
     if (B <= 0) return set_err(h, LDEQ_ERR_INVALID, "B must be > 0");
     cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = refuse_capture(h, s, "ldeq_solve_fwd_bwd_host", "it stages through host memory and synchronises the stream"))) return rc;
     LDEQ_CUDA(cudaSetDevice(h->device));
     if ((rc = host_streams(h))) return rc;
     const size_t es = dtype == LDEQ_F32 ? 4 : 8, zb = (size_t)rhs->z_dim * es, pb = (size_t)rhs->p_dim * es;
     const size_t nz = (size_t)B * zb, np = (size_t)B * pb, nt = nz * (size_t)T;
     HostBufs hb;
-    if ((rc = host_bufs(h, nz, np, nt, B, true, true, &hb))) return rc;
+    if ((rc = host_bufs(h, nz, np, nt, B, true, true, &hb, s))) return rc;
     if ((rc = upload_tgrid(h, t_host, T, s))) return rc;
     LDEQ_CUDA(cudaMemcpyAsync(hb.z0, z0_host, nz, cudaMemcpyHostToDevice, s));
     LDEQ_CUDA(cudaMemcpyAsync(hb.th, theta_host, np, cudaMemcpyHostToDevice, s));
@@ -730,7 +842,7 @@ int ldeq_solve_fwd_bwd_host(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, cons
         slab_bounds(B, ns, i, &b0, &nb);
         if (nb <= 0) continue;
         ldeq_tape* part = nullptr;
-        rc = solve_fwd_slab(h, rhs, dtype, hb.z0 + b0 * zb, hb.th + b0 * pb, t_host, nb, B, T, opts, hb.traj + b0 * zb, hb.ret + b0,
+        rc = solve_fwd_slab(h, rhs, dtype, hb.z0 + b0 * zb, hb.th + b0 * pb, t_host, eager_grid(h), false, nb, B, T, opts, hb.traj + b0 * zb, hb.ret + b0,
                             hb.na + b0, hb.nr + b0, &part, s);
         if (rc) return rc;
         LDEQ_CUDA(cudaEventRecord(h->ev_fwd[i], s));
@@ -740,7 +852,7 @@ int ldeq_solve_fwd_bwd_host(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, cons
         LDEQ_CUDA(cudaStreamWaitEvent(s, h->ev_up[i], 0));
         rc = solve_bwd_slab(h, part, hb.dtraj + b0 * zb, B, hb.dz0 + b0 * zb, hb.dth + b0 * pb, s);
         cudaFreeAsync(part->base, s);
-        slot_put(h, part);
+        slot_put(h, part, s);
         delete part;
         if (rc) return rc;
     }

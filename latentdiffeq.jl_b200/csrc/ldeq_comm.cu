@@ -77,6 +77,7 @@ int ldeq_comm_init(ldeq_handle* h, const void* unique_id, int rank, int nranks) 
 
 int ldeq_allreduce_grads(ldeq_handle* h, float* grads_flat, int64_t n, ldeq_stream stream) {
     if (!h) return LDEQ_ERR_INVALID;
+    if (int rc = ldeq::refuse_capture(h, (cudaStream_t)stream, "ldeq_allreduce_grads", "multi-GPU capture is not supported")) return rc;
     if (!h->nccl_comm) return ldeq::set_err(h, LDEQ_ERR_INVALID, "allreduce_grads: call ldeq_comm_init first");
     if (!grads_flat || n < 0) return ldeq::set_err(h, LDEQ_ERR_INVALID, "allreduce_grads: bad buffer");
     if (n == 0) return LDEQ_OK;

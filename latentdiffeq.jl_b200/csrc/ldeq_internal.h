@@ -11,6 +11,7 @@
 #include "ldeq_common.cuh"
 
 #define LDEQ_MAX_SLABS 8  // column slabs a host-resident batch is cut into (ldeq_api.cu)
+#define LDEQ_GRID_CACHE 16  // unpinned immutable grid copies a handle keeps (ldeq_handle::grid_cache)
 
 struct ldeq_handle {
     int device = 0;
@@ -23,9 +24,26 @@ struct ldeq_handle {
     // the cached grid is t0 + k*h bit for bit (checked on upload): kernels then compute save times instead of looking them up
     double grid_t0 = 0.0, grid_h = 0.0;
     int grid_uniform = 0;
+    // Grids a captured CUDA graph may read: d_tgrid above is overwritten in place when a call brings another grid, so a
+    // solve under stream capture reads an immutable device copy from this cache instead.  Every eager upload of a new grid
+    // adds one (the most recent LDEQ_GRID_CACHE unpinned ones are kept); a capture pins the entry it reads, and pinned
+    // entries live until ldeq_destroy.
+    struct GridEntry {
+        std::vector<double> t;
+        double* d = nullptr;
+        double t0 = 0.0, h = 0.0;
+        int uniform = 0;
+        bool pinned = false;
+        uint64_t last_use = 0;
+    };
+    std::vector<GridEntry> grid_cache;
+    uint64_t grid_clock = 0;
     // grow-only device scratch for the *_host entry points and reductions
     void* scratch[4] = {nullptr, nullptr, nullptr, nullptr};
     size_t scratch_cap[4] = {0, 0, 0, 0};
+    // a scratch slot that a capture has referenced is retired (kept until ldeq_destroy) instead of freed when it grows
+    bool scratch_captured[4] = {false, false, false, false};
+    std::vector<void*> retired_scratch;
     // ELBO reduction workspace
     double* d_partials = nullptr;
     unsigned int* d_counter = nullptr;
@@ -35,6 +53,7 @@ struct ldeq_handle {
     // recycled {pinned info slot, event} pairs for tapes (cudaMallocHost / cudaEventCreate are slow)
     struct Slot { int32_t* h_info; cudaEvent_t ev; };
     std::vector<Slot> free_slots;
+    std::vector<Slot> deferred_slots;  // released under capture: returned to free_slots by the next slot_acquire
     std::vector<int32_t*> pinned_blocks;
     // NCCL communicator of the gradient all-reduce (ldeq_comm.cu; libnccl is dlopen'ed on first use)
     void* nccl_lib = nullptr;
@@ -86,8 +105,14 @@ struct ldeq_tape {
 namespace ldeq {
 
 int set_err(ldeq_handle* h, int code, const char* what, cudaError_t ce = cudaSuccess);
+// True while `s` is being captured into a CUDA graph (or its capture was invalidated): work enqueued now is recorded, not
+// run, so the host can neither wait for it nor read its results, and every pointer it reads is frozen into the graph.
+bool capturing(cudaStream_t s);
+// LDEQ_ERR_UNSUPPORTED with "<what>: not available under CUDA graph capture (<why>)" when `s` is capturing, else LDEQ_OK.
+int refuse_capture(ldeq_handle* h, cudaStream_t s, const char* what, const char* why);
 int upload_tgrid(ldeq_handle* h, const double* t_host, int T, cudaStream_t s);
-int ensure_scratch(ldeq_handle* h, int slot, size_t bytes);
+// grows scratch[slot] to `bytes` on `s`; under capture it refuses to grow (LDEQ_ERR_UNSUPPORTED) and marks the slot captured
+int ensure_scratch(ldeq_handle* h, int slot, size_t bytes, cudaStream_t s);
 KOpts to_kopts(const ldeq_opts* o);
 int bwd_sort_lanes();  // ldeq_api.cu: lane re-deal of the discrete-adjoint kernels (LDEQ_BWD_SORT)
 // pooled pinned {int32 x 2} mirror + event (ldeq_api.cu)

@@ -44,8 +44,13 @@ struct KlHeads {
 // (summed in index order by the last block of elbo_mse_kernel: deterministic).  One block used to do all of it: 0.53 ms
 // at B = 8192 (ncu, profiles/r2_loss_kernels_summary.txt) -- as long as the 1.3 GB reconstruction term next to it.
 #define ELBO_KL_BLOCKS 64
-__global__ void __launch_bounds__(ELBO_THREADS) elbo_kl_kernel(KlHeads hd, int B, float gscale_beta, double* __restrict__ kl_partials) {
+// DEV: beta is read from beta_dev (a CUDA graph replays it with new values) and gscale_beta = gscale * beta is formed here,
+// in the same Float32 rounding as the host forms it for DEV = false
+template <bool DEV>
+__global__ void __launch_bounds__(ELBO_THREADS) elbo_kl_kernel(KlHeads hd, int B, float gscale_beta, const float* __restrict__ beta_dev,
+                                                               double* __restrict__ kl_partials) {
     __shared__ double sh[ELBO_THREADS / 32];
+    if (DEV) gscale_beta = __fmul_rn(gscale_beta, *beta_dev);
     double acc = 0.0;
     const float invB = 1.0f / (float)B;
     for (int hI = 0; hI < hd.n_heads; ++hI) {
@@ -76,11 +81,11 @@ __global__ void __launch_bounds__(ELBO_THREADS) elbo_kl_kernel(KlHeads hd, int B
 // its backward pass and the x-hat round trip through HBM between them and the loss never exist.
 __device__ __forceinline__ float elbo_sigmoid(float a) { return 1.0f / (1.0f + expf(-a)); }
 
-template <bool GRAD, bool LOGITS>
+template <bool GRAD, bool LOGITS, bool DEV>
 __global__ void __launch_bounds__(ELBO_THREADS)
 elbo_mse_kernel(const float* __restrict__ x, const float* __restrict__ xhat, float* __restrict__ dxhat, size_t n,
-                float inv_bt, float gscale, float beta, double* __restrict__ partials, unsigned int* __restrict__ counter,
-                const double* __restrict__ kl_partials, int n_kl, float* __restrict__ loss) {
+                float inv_bt, float gscale, float beta, const float* __restrict__ beta_dev, double* __restrict__ partials,
+                unsigned int* __restrict__ counter, const double* __restrict__ kl_partials, int n_kl, float* __restrict__ loss) {
     __shared__ float shw[ELBO_THREADS / 32];
     __shared__ bool is_last;
     const size_t n4 = n >> 2;
@@ -137,6 +142,7 @@ elbo_mse_kernel(const float* __restrict__ x, const float* __restrict__ xhat, flo
             double klsum = 0.0;
             for (int i = 0; i < n_kl; ++i) klsum += __ldcg(kl_partials + i);   // written by the preceding elbo_kl_kernel
             const float klf = (float)klsum;
+            if (DEV) beta = *beta_dev;
             loss[1] = rec;
             loss[2] = klf;
             loss[0] = rec + beta * klf;
@@ -158,9 +164,16 @@ __device__ __forceinline__ void adamw_one(float& x, float g, float& m, float& v,
     x = x - d;
 }
 
+// DEV: the bias corrections come from the device state that adamw_advance_kernel has just advanced
+template <bool DEV>
 __global__ void __launch_bounds__(256)
 adamw_kernel(float* __restrict__ x, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, size_t n,
-             double b1, double b2, double c1, double c2, double eps, double lr, float decay, float gscale) {
+             double b1, double b2, double c1, double c2, double eps, double lr, float decay, float gscale,
+             const ldeq_adamw_state* __restrict__ state) {
+    if (DEV) {
+        c1 = 1.0 - state->beta1_pow;
+        c2 = 1.0 - state->beta2_pow;
+    }
     const size_t n4 = n >> 2;
     float4* x4 = reinterpret_cast<float4*>(x);
     const float4* g4 = reinterpret_cast<const float4*>(g);
@@ -181,6 +194,14 @@ adamw_kernel(float* __restrict__ x, const float* __restrict__ g, float* __restri
         adamw_one(xx, g[i] * gscale, mm, vv, b1, b2, c1, c2, eps, lr, decay);
         x[i] = xx; m[i] = mm; v[i] = vv;
     }
+}
+
+// One thread: the next step of the running Float64 beta powers, the same multiplications in the same order as the host loop
+// of ldeq_adamw_step.  A launch of its own, so that every CTA of the update reads the state after it has advanced.
+__global__ void adamw_advance_kernel(ldeq_adamw_state* state, double b1, double b2) {
+    state->step += 1;
+    state->beta1_pow *= b1;
+    state->beta2_pow *= b2;
 }
 
 // ---- all-reduce fused with AdamW over peer memory ----------------------------------------------------------------
@@ -253,9 +274,12 @@ __device__ __forceinline__ void box_muller(uint32_t a, uint32_t b, float* n0, fl
 }
 
 // each thread produces 4 normals (one Philox block) for elements 4i..4i+3
+// DEV: offset = *calls << 32, from the counter sample_advance_kernel has just incremented
+template <bool DEV>
 __global__ void __launch_bounds__(256)
 sample_kernel(const float* __restrict__ mu, const float* __restrict__ lv, float* __restrict__ z, float* __restrict__ eps,
-              size_t n, uint64_t seed, uint64_t offset) {
+              size_t n, uint64_t seed, uint64_t offset, const uint64_t* __restrict__ calls) {
+    if (DEV) offset = *calls << 32;
     const size_t nb = (n + 3) >> 2;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nb; i += stride) {
@@ -276,15 +300,18 @@ sample_kernel(const float* __restrict__ mu, const float* __restrict__ lv, float*
     }
 }
 
+__global__ void sample_advance_kernel(uint64_t* calls) { *calls += 1; }
+
 }  // namespace ldeq
 
 using namespace ldeq;
 
 extern "C" {
 
+// beta_dev != null: the _dev variants, beta is read on the device
 static int elbo_impl(bool logits, ldeq_handle* h, const float* x, const float* xhat, const float* const* mu_host,
-                     const float* const* logvar_host, const int32_t* head_dims_host, int n_heads, float beta, int B,
-                     int T, int P, float grad_scale, float* loss, float* dxhat, float* const* dmu_host,
+                     const float* const* logvar_host, const int32_t* head_dims_host, int n_heads, float beta, const float* beta_dev,
+                     int B, int T, int P, float grad_scale, float* loss, float* dxhat, float* const* dmu_host,
                      float* const* dlogvar_host, ldeq_stream stream) {
     if (!h) return LDEQ_ERR_INVALID;
     if (!x || !xhat || !loss || n_heads < 0 || n_heads > 4 || B <= 0 || T <= 0 || P <= 0)
@@ -295,6 +322,9 @@ static int elbo_impl(bool logits, ldeq_handle* h, const float* x, const float* x
     LDEQ_CUDA(cudaSetDevice(h->device));
     const int max_blocks = h->sm_count * 8;
     if (!h->d_partials) {
+        if (capturing(s))
+            return set_err(h, LDEQ_ERR_UNSUPPORTED, "elbo: the reduction workspace is allocated by the first call, which cannot happen under "
+                                                    "CUDA graph capture: call the loss once outside the capture first");
         LDEQ_CUDA(cudaMalloc((void**)&h->d_partials, sizeof(double) * (max_blocks + ELBO_KL_BLOCKS)));
         LDEQ_CUDA(cudaMalloc((void**)&h->d_counter, sizeof(unsigned int)));
         LDEQ_CUDA(cudaMemset(h->d_counter, 0, sizeof(unsigned int)));
@@ -315,15 +345,18 @@ static int elbo_impl(bool logits, ldeq_handle* h, const float* x, const float* x
     int kl_grid = 1;
     for (int i = 0; i < n_heads; ++i) { const int w = (hd.n[i] + 4 * ELBO_THREADS - 1) / (4 * ELBO_THREADS); if (w > kl_grid) kl_grid = w; }
     if (kl_grid > ELBO_KL_BLOCKS) kl_grid = ELBO_KL_BLOCKS;
-    elbo_kl_kernel<<<kl_grid, ELBO_THREADS, 0, s>>>(hd, B, grad_scale * beta, kl_partials);
+    if (beta_dev) elbo_kl_kernel<true><<<kl_grid, ELBO_THREADS, 0, s>>>(hd, B, grad_scale, beta_dev, kl_partials);
+    else elbo_kl_kernel<false><<<kl_grid, ELBO_THREADS, 0, s>>>(hd, B, grad_scale * beta, nullptr, kl_partials);
     LDEQ_CUDA(cudaGetLastError());
     const size_t n = (size_t)P * B * T;
     size_t want = ((n >> 2) + ELBO_THREADS - 1) / ELBO_THREADS;
     int grid = (int)(want < (size_t)max_blocks ? (want ? want : 1) : (size_t)max_blocks);
     const float inv_bt = 1.0f / ((float)B * (float)T);
-#define LDEQ_ELBO_LAUNCH(G, L) elbo_mse_kernel<G, L><<<grid, ELBO_THREADS, 0, s>>>(x, xhat, dxhat, n, inv_bt, grad_scale, beta, h->d_partials, h->d_counter, kl_partials, kl_grid, loss)
-    if (dxhat) { if (logits) LDEQ_ELBO_LAUNCH(true, true); else LDEQ_ELBO_LAUNCH(true, false); }
-    else { if (logits) LDEQ_ELBO_LAUNCH(false, true); else LDEQ_ELBO_LAUNCH(false, false); }
+#define LDEQ_ELBO_LAUNCH(G, L, D) elbo_mse_kernel<G, L, D><<<grid, ELBO_THREADS, 0, s>>>(x, xhat, dxhat, n, inv_bt, grad_scale, beta, beta_dev, h->d_partials, h->d_counter, kl_partials, kl_grid, loss)
+#define LDEQ_ELBO_LAUNCH_D(G, L) do { if (beta_dev) LDEQ_ELBO_LAUNCH(G, L, true); else LDEQ_ELBO_LAUNCH(G, L, false); } while (0)
+    if (dxhat) { if (logits) LDEQ_ELBO_LAUNCH_D(true, true); else LDEQ_ELBO_LAUNCH_D(true, false); }
+    else { if (logits) LDEQ_ELBO_LAUNCH_D(false, true); else LDEQ_ELBO_LAUNCH_D(false, false); }
+#undef LDEQ_ELBO_LAUNCH_D
 #undef LDEQ_ELBO_LAUNCH
     LDEQ_CUDA(cudaGetLastError());
     h->launches += 2;
@@ -334,7 +367,16 @@ int ldeq_elbo_fwd_bwd(ldeq_handle* h, const float* x, const float* xhat, const f
                       const float* const* logvar_host, const int32_t* head_dims_host, int n_heads, float beta, int B,
                       int T, int P, float grad_scale, float* loss, float* dxhat, float* const* dmu_host,
                       float* const* dlogvar_host, ldeq_stream stream) {
-    return elbo_impl(false, h, x, xhat, mu_host, logvar_host, head_dims_host, n_heads, beta, B, T, P, grad_scale, loss, dxhat, dmu_host,
+    return elbo_impl(false, h, x, xhat, mu_host, logvar_host, head_dims_host, n_heads, beta, nullptr, B, T, P, grad_scale, loss, dxhat, dmu_host,
+                     dlogvar_host, stream);
+}
+
+int ldeq_elbo_fwd_bwd_dev(ldeq_handle* h, const float* x, const float* xhat, const float* const* mu_host,
+                          const float* const* logvar_host, const int32_t* head_dims_host, int n_heads, const float* beta, int B,
+                          int T, int P, float grad_scale, float* loss, float* dxhat, float* const* dmu_host,
+                          float* const* dlogvar_host, ldeq_stream stream) {
+    if (h && !beta) return set_err(h, LDEQ_ERR_INVALID, "elbo: null beta");
+    return elbo_impl(false, h, x, xhat, mu_host, logvar_host, head_dims_host, n_heads, 0.0f, beta, B, T, P, grad_scale, loss, dxhat, dmu_host,
                      dlogvar_host, stream);
 }
 
@@ -342,7 +384,16 @@ int ldeq_elbo_logits_fwd_bwd(ldeq_handle* h, const float* x, const float* logits
                              const float* const* logvar_host, const int32_t* head_dims_host, int n_heads, float beta, int B,
                              int T, int P, float grad_scale, float* loss, float* dlogits, float* const* dmu_host,
                              float* const* dlogvar_host, ldeq_stream stream) {
-    return elbo_impl(true, h, x, logits, mu_host, logvar_host, head_dims_host, n_heads, beta, B, T, P, grad_scale, loss, dlogits, dmu_host,
+    return elbo_impl(true, h, x, logits, mu_host, logvar_host, head_dims_host, n_heads, beta, nullptr, B, T, P, grad_scale, loss, dlogits, dmu_host,
+                     dlogvar_host, stream);
+}
+
+int ldeq_elbo_logits_fwd_bwd_dev(ldeq_handle* h, const float* x, const float* logits, const float* const* mu_host,
+                                 const float* const* logvar_host, const int32_t* head_dims_host, int n_heads, const float* beta, int B,
+                                 int T, int P, float grad_scale, float* loss, float* dlogits, float* const* dmu_host,
+                                 float* const* dlogvar_host, ldeq_stream stream) {
+    if (h && !beta) return set_err(h, LDEQ_ERR_INVALID, "elbo: null beta");
+    return elbo_impl(true, h, x, logits, mu_host, logvar_host, head_dims_host, n_heads, 0.0f, beta, B, T, P, grad_scale, loss, dlogits, dmu_host,
                      dlogvar_host, stream);
 }
 
@@ -362,7 +413,29 @@ int ldeq_adamw_step(ldeq_handle* h, float* params, const float* grads, float* m,
     for (int64_t i = 0; i < step; ++i) { p1 *= b1; p2 *= b2; }
     size_t want = (((size_t)n >> 2) + 255) / 256;
     int grid = (int)(want < (size_t)h->sm_count * 8 ? (want ? want : 1) : (size_t)h->sm_count * 8);
-    adamw_kernel<<<grid, 256, 0, s>>>(params, grads, m, v, (size_t)n, b1, b2, 1.0 - p1, 1.0 - p2, epsd, lrd, decay, grad_scale);
+    adamw_kernel<false><<<grid, 256, 0, s>>>(params, grads, m, v, (size_t)n, b1, b2, 1.0 - p1, 1.0 - p2, epsd, lrd, decay, grad_scale, nullptr);
+    LDEQ_CUDA(cudaGetLastError());
+    h->launches += 1;
+    return LDEQ_OK;
+}
+
+int ldeq_adamw_step_dev(ldeq_handle* h, float* params, const float* grads, float* m, float* v, int64_t n, double lr,
+                        double beta1, double beta2, double eps, float decay, ldeq_adamw_state* state, float grad_scale,
+                        ldeq_stream stream) {
+    if (!h) return LDEQ_ERR_INVALID;
+    if (!params || !grads || !m || !v || !state || n < 0) return set_err(h, LDEQ_ERR_INVALID, "adamw: bad argument");
+    if ((((uintptr_t)params) | ((uintptr_t)grads) | ((uintptr_t)m) | ((uintptr_t)v)) & 15)
+        return set_err(h, LDEQ_ERR_INVALID, "adamw: buffers must be 16-byte aligned");
+    if ((uintptr_t)state & 7) return set_err(h, LDEQ_ERR_INVALID, "adamw: state must be 8-byte aligned");
+    cudaStream_t s = (cudaStream_t)stream;
+    LDEQ_CUDA(cudaSetDevice(h->device));
+    adamw_advance_kernel<<<1, 1, 0, s>>>(state, beta1, beta2);
+    LDEQ_CUDA(cudaGetLastError());
+    h->launches += 1;
+    if (n == 0) return LDEQ_OK;
+    size_t want = (((size_t)n >> 2) + 255) / 256;
+    int grid = (int)(want < (size_t)h->sm_count * 8 ? (want ? want : 1) : (size_t)h->sm_count * 8);
+    adamw_kernel<true><<<grid, 256, 0, s>>>(params, grads, m, v, (size_t)n, beta1, beta2, 0.0, 0.0, eps, lr, decay, grad_scale, state);
     LDEQ_CUDA(cudaGetLastError());
     h->launches += 1;
     return LDEQ_OK;
@@ -389,8 +462,9 @@ int ldeq_allreduce_adamw_step(ldeq_handle* h, float* params, float* const* peer_
         al |= (uintptr_t)pb.g[r] | (uintptr_t)pb.x[r];
     }
     if (al & 15) return set_err(h, LDEQ_ERR_INVALID, "allreduce_adamw: buffers must be 16-byte aligned");
-    if (n == 0) return LDEQ_OK;
     cudaStream_t s = (cudaStream_t)stream;
+    if (int rc = refuse_capture(h, s, "ldeq_allreduce_adamw_step", "multi-GPU capture is not supported")) return rc;
+    if (n == 0) return LDEQ_OK;
     LDEQ_CUDA(cudaSetDevice(h->device));
     double p1 = 1.0, p2 = 1.0;
     for (int64_t i = 0; i < step; ++i) { p1 *= beta1; p2 *= beta2; }
@@ -421,7 +495,26 @@ int ldeq_sample(ldeq_handle* h, const float* mu, const float* logvar, float* z_o
     LDEQ_CUDA(cudaSetDevice(h->device));
     size_t want = ((((size_t)n + 3) >> 2) + 255) / 256;
     int grid = (int)(want < (size_t)h->sm_count * 8 ? want : (size_t)h->sm_count * 8);
-    sample_kernel<<<grid, 256, 0, s>>>(mu, logvar, z_out, eps_out, (size_t)n, seed, offset);
+    sample_kernel<false><<<grid, 256, 0, s>>>(mu, logvar, z_out, eps_out, (size_t)n, seed, offset, nullptr);
+    LDEQ_CUDA(cudaGetLastError());
+    h->launches += 1;
+    return LDEQ_OK;
+}
+
+int ldeq_sample_dev(ldeq_handle* h, const float* mu, const float* logvar, float* z_out, float* eps_out, int64_t n,
+                    uint64_t seed, uint64_t* calls, ldeq_stream stream) {
+    if (!h) return LDEQ_ERR_INVALID;
+    if (!mu || !logvar || !z_out || !calls || n < 0) return set_err(h, LDEQ_ERR_INVALID, "sample: bad argument");
+    if ((uintptr_t)calls & 7) return set_err(h, LDEQ_ERR_INVALID, "sample: calls must be 8-byte aligned");
+    cudaStream_t s = (cudaStream_t)stream;
+    LDEQ_CUDA(cudaSetDevice(h->device));
+    sample_advance_kernel<<<1, 1, 0, s>>>(calls);
+    LDEQ_CUDA(cudaGetLastError());
+    h->launches += 1;
+    if (n == 0) return LDEQ_OK;
+    size_t want = ((((size_t)n + 3) >> 2) + 255) / 256;
+    int grid = (int)(want < (size_t)h->sm_count * 8 ? want : (size_t)h->sm_count * 8);
+    sample_kernel<true><<<grid, 256, 0, s>>>(mu, logvar, z_out, eps_out, (size_t)n, seed, 0, calls);
     LDEQ_CUDA(cudaGetLastError());
     h->launches += 1;
     return LDEQ_OK;

@@ -432,7 +432,7 @@ static int mlp_fwd_dispatch(ldeq_handle* h, const MlpNet& net, const void* P, co
     MlpTapeView<S> tv{nullptr, nullptr, nullptr, 0};
     if (tape) tv = MlpTapeView<S>{tape->t, tape->dt, (S*)tape->u, tape->cap};
     // reduction scratch for the grid sums
-    int rc = ensure_scratch(h, 0, sizeof(double) * 4096);
+    int rc = ensure_scratch(h, 0, sizeof(double) * 4096, s);
     if (rc) return rc;
     double* partials = (double*)h->scratch[0];
     const int sms = h->sm_count;
@@ -479,6 +479,7 @@ int ldeq_mlp_solve_fwd(ldeq_handle* h, int dtype, const void* z0, const void* pa
                        ldeq_stream stream) {
     if (!h) return LDEQ_ERR_INVALID;
     if (tape_out) *tape_out = nullptr;
+    if (int rc0 = refuse_capture(h, (cudaStream_t)stream, "ldeq_mlp_solve_fwd", "its tape records the accepted-step count for a host-side check")) return rc0;
     if (!z0 || !params_flat || !layer_dims_host || !t_host || !opts || !traj_out) return set_err(h, LDEQ_ERR_INVALID, "null argument");
     if (B < 1 || T < 1) return set_err(h, LDEQ_ERR_INVALID, "B and T must be >= 1");
     if (dtype != LDEQ_F32 && dtype != LDEQ_F64) return set_err(h, LDEQ_ERR_INVALID, "dtype");
@@ -578,7 +579,7 @@ static int launch_mlp_bwd(ldeq_handle* h, ldeq_mlp_tape* tape, const void* dtraj
     const bool smem_grad = smem_g <= 225 * 1024 && tiles <= h->sm_count;
     const int per_sm = smem_grad ? 1 : 2;
     const int grid = tiles < per_sm * h->sm_count ? tiles : per_sm * h->sm_count;
-    int rc = ensure_scratch(h, 1, (size_t)grid * net.n_params * sizeof(S));
+    int rc = ensure_scratch(h, 1, (size_t)grid * net.n_params * sizeof(S), s);
     if (rc) return rc;
     mlp_transpose_kernel<S><<<64, 256, 0, s>>>(net, (const S*)tape->params, (S*)tape->params_t);
     // biases are not used from the transposed copy
@@ -634,14 +635,14 @@ static int launch_mlp_cadj(ldeq_handle* h, ldeq_mlp_tape* tape, const void* dtra
     const size_t NP = net.n_params, D = net.dims[0];
     const int na = tape->h_info[0] > 0 ? tape->h_info[0] : 1;
     int rc;
-    if ((rc = ensure_scratch(h, 0, sizeof(double) * 4096))) return rc;
-    if ((rc = ensure_scratch(h, 1, (size_t)grid * 2 * NP * sizeof(S)))) return rc;
+    if ((rc = ensure_scratch(h, 0, sizeof(double) * 4096, s))) return rc;
+    if ((rc = ensure_scratch(h, 1, (size_t)grid * 2 * NP * sizeof(S), s))) return rc;
     const size_t dense_bytes = ((size_t)na * 7 * D * grid * TB * sizeof(S) + 255) & ~(size_t)255;
     const size_t grec_bytes = res ? (size_t)grid * 7 * CadjRec<S, TB>::floats(net.dims[0], net.max_width, net.n_layers) * sizeof(S) : 0;
-    if ((rc = ensure_scratch(h, 3, dense_bytes + grec_bytes))) return rc;
+    if ((rc = ensure_scratch(h, 3, dense_bytes + grec_bytes, s))) return rc;
     const size_t mu_bytes = (3 * NP * sizeof(S) + 255) & ~(size_t)255;
     const int trace_cap = getenv("LDEQ_CADJ_TRACE") ? 4096 : 0;  // debugging aid: (t, dt, EEst, accept) of every attempt
-    if ((rc = ensure_scratch(h, 2, mu_bytes + (size_t)trace_cap * 32 + 256))) return rc;
+    if ((rc = ensure_scratch(h, 2, mu_bytes + (size_t)trace_cap * 32 + 256, s))) return rc;
     mlp_transpose_kernel<S><<<64, 256, 0, s>>>(net, (const S*)tape->params, (S*)tape->params_t);
     LDEQ_CUDA(cudaGetLastError());
     MlpNet netv = net;
@@ -693,6 +694,7 @@ int ldeq_mlp_solve_bwd(ldeq_handle* h, ldeq_mlp_tape* tape, const void* dtraj, v
     if (!h) return LDEQ_ERR_INVALID;
     if (!tape || !dtraj || !dz0 || !dparams_flat) return set_err(h, LDEQ_ERR_INVALID, "null argument");
     cudaStream_t s = (cudaStream_t)stream;
+    if (int rc0 = refuse_capture(h, s, "ldeq_mlp_solve_bwd", "it waits for the forward kernel to check the tape for overflow on the host")) return rc0;
     LDEQ_CUDA(cudaSetDevice(h->device));
     // a solve that took more accepted steps than the tape holds has no exact gradient: say so instead of returning
     // NaN / partial sums (waits for the forward kernel, as the GOKU path's tape check does)
@@ -750,6 +752,7 @@ int ldeq_debug_cadj_trace(ldeq_handle* h, ldeq_mlp_tape* tape, double* out_host,
 int ldeq_mlp_bwd_stats(ldeq_handle* h, ldeq_mlp_tape* tape, int32_t* out3_host, ldeq_stream stream) {
     if (!h) return LDEQ_ERR_INVALID;
     if (!tape || !out3_host) return set_err(h, LDEQ_ERR_INVALID, "null argument");
+    if (int rc0 = refuse_capture(h, (cudaStream_t)stream, "ldeq_mlp_bwd_stats", "it synchronises the stream")) return rc0;
     LDEQ_CUDA(cudaSetDevice(h->device));
     LDEQ_CUDA(cudaMemcpyAsync(out3_host, tape->info + 4, 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
     LDEQ_CUDA(cudaStreamSynchronize((cudaStream_t)stream));

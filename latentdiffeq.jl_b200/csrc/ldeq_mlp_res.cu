@@ -398,7 +398,7 @@ int ldeq_mlp_res_backward(ldeq_handle* h, const MlpNet& net, const float* P, con
     const int tiles = (B + TB - 1) / TB;
     if (tiles > 4 * h->sm_count) return LDEQ_ERR_UNSUPPORTED;  // many rounds of tiles: the general kernel's 2 CTAs per SM win
     const int grid = tiles < h->sm_count ? tiles : h->sm_count;
-    int rc = ensure_scratch(h, 1, (size_t)grid * net.n_params * sizeof(float));
+    int rc = ensure_scratch(h, 1, (size_t)grid * net.n_params * sizeof(float), s);
     if (rc) return rc;
     LDEQ_CUDA(cudaFuncSetAttribute(mlp_bwd_res_kernel<TB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     MlpNet netv = net;

@@ -436,9 +436,9 @@ int ldeq_mlp_tc_forward(ldeq_handle* h, const int32_t* dims, int n_layers, const
     int rc = ldeq_tc_make_net(h, dims, n_layers, &net);
     if (rc) return rc;
     const int D = dims[0], H1 = dims[1], H2 = dims[2];
-    rc = ensure_scratch(h, 2, (size_t)net.smem_bytes);
+    rc = ensure_scratch(h, 2, (size_t)net.smem_bytes, s);
     if (rc) return rc;
-    rc = ensure_scratch(h, 0, sizeof(double) * 4096);
+    rc = ensure_scratch(h, 0, sizeof(double) * 4096, s);
     if (rc) return rc;
     unsigned char* img = (unsigned char*)h->scratch[2];
     mlp_tc_prep_kernel<<<64, 256, 0, s>>>(net, params, D, H1, H2, img);

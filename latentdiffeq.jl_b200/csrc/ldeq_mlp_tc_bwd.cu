@@ -637,9 +637,9 @@ int ldeq_mlp_tc_backward(ldeq_handle* h, const int32_t* dims, int n_layers, cons
     const int wg_grid = h->sm_count;
     const size_t part_floats = (size_t)net.n2 * net.n1 + (size_t)net.n1 * TC_G_FEATS + (size_t)net.n2 * TC_D_FEATS;
     // scratch: [2] weight images, [1] records + tile step counts, [3] per-CTA partial gradients
-    if ((rc = ensure_scratch(h, 2, (size_t)net.smem_bytes))) return rc;
-    if ((rc = ensure_scratch(h, 1, rec_bytes + (size_t)tiles * sizeof(int) + 256))) return rc;
-    if ((rc = ensure_scratch(h, 3, (size_t)wg_grid * part_floats * sizeof(float)))) return rc;
+    if ((rc = ensure_scratch(h, 2, (size_t)net.smem_bytes, s))) return rc;
+    if ((rc = ensure_scratch(h, 1, rec_bytes + (size_t)tiles * sizeof(int) + 256, s))) return rc;
+    if ((rc = ensure_scratch(h, 3, (size_t)wg_grid * part_floats * sizeof(float), s))) return rc;
     unsigned char* img = (unsigned char*)h->scratch[2];
     unsigned char* records = (unsigned char*)h->scratch[1];
     int* tile_nsteps = (int*)(records + ((rec_bytes + 255) & ~(size_t)255));

@@ -17,6 +17,7 @@ the bytes are identical: Julia ``(features, batch, time)`` is torch ``[time, bat
 """
 from __future__ import annotations
 
+import contextlib
 import math
 
 import torch
@@ -265,23 +266,38 @@ def apply_latent_in(encoder, pe_out):
 
 
 _sample_calls = 0
+_sample_counter = None
+
+
+@contextlib.contextmanager
+def device_sample_counter(calls: torch.Tensor):
+    """Inside the block ``sample`` draws through ``ldeq_sample_dev`` with the device counter ``calls`` (one int64 element that
+    mirrors ``_sample_calls``): a captured CUDA graph then draws new noise on every replay.  The host counter still advances
+    once per draw, as it does outside the block."""
+    global _sample_counter
+    prev, _sample_counter = _sample_counter, calls
+    try:
+        yield
+    finally:
+        _sample_counter = prev
 
 
 def sample(mu, logvar, model, seed: int | None = None):
     """Reparameterised sample ``mu + eps * exp(logvar/2)`` (GOKU.jl:155-173, LatentODE.jl:82-98).
     The noise is drawn on the device by ``ldeq_sample`` (the reference draws it on the host and
     uploads it, GOKU.jl:169-170)."""
-    global _sample_calls
     if seed is None:
         seed = int(torch.initial_seed() & 0x7FFFFFFFFFFFFFFF)
+
+    def draw(m, lv):
+        global _sample_calls
+        _sample_calls += 1
+        if _sample_counter is None:
+            return sample_reparam(m, lv, seed, _sample_calls << 32)
+        return sample_reparam(m, lv, seed, _sample_calls << 32, _sample_counter)
     if isinstance(mu, tuple):
-        out = []
-        for m, lv in zip(mu, logvar):
-            _sample_calls += 1
-            out.append(sample_reparam(m, lv, seed, _sample_calls << 32))
-        return tuple(out)
-    _sample_calls += 1
-    return sample_reparam(mu, logvar, seed, _sample_calls << 32)
+        return tuple(draw(m, lv) for m, lv in zip(mu, logvar))
+    return draw(mu, logvar)
 
 
 def apply_latent_out(decoder, l_tilde):
@@ -344,13 +360,21 @@ def apply_reconstructor(decoder, z_hat):
     return decoder.reconstructor(z_hat)
 
 
+def _logits_layers(decoder):
+    """The reconstructor's layers when its last one is a ``Dense`` with the sigmoid output activation, else ``None``."""
+    rec = decoder.reconstructor
+    layers = list(rec) if isinstance(rec, nn.Sequential) else []
+    if not layers or not isinstance(layers[-1], Dense) or layers[-1].act is not torch.sigmoid:
+        return None
+    return layers
+
+
 def reconstructor_logits(decoder, z_hat):
     """The reconstructor up to the pre-activations of its last layer, when that layer is a ``Dense`` with the sigmoid output
     activation of ``default_layers`` (GOKU.jl:265-268); ``None`` otherwise.  ``ldeq_elbo_logits_fwd_bwd`` applies the sigmoid
     inside the loss kernel."""
-    rec = decoder.reconstructor
-    layers = list(rec) if isinstance(rec, nn.Sequential) else []
-    if not layers or not isinstance(layers[-1], Dense) or layers[-1].act is not torch.sigmoid:
+    layers = _logits_layers(decoder)
+    if layers is None:
         return None
     h = z_hat
     for l in layers[:-1]:

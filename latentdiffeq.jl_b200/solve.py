@@ -446,43 +446,51 @@ def pattern_extractor(x: torch.Tensor, rnn_layers, lstm_f_layers=None, lstm_b_la
 
 
 # ---- reparameterised sample, ELBO, AdamW ------------------------------------------------------------
-def sample_raw(mu: torch.Tensor, logvar: torch.Tensor, seed: int, offset: int = 0, want_eps: bool = True):
-    """``ldeq_sample``: ``z = mu + eps * exp(logvar/2)``, ``eps ~ N(0,1)`` drawn on the device (Philox4x32-10)."""
+def sample_raw(mu: torch.Tensor, logvar: torch.Tensor, seed: int, offset: int = 0, want_eps: bool = True,
+               calls: torch.Tensor | None = None):
+    """``ldeq_sample``: ``z = mu + eps * exp(logvar/2)``, ``eps ~ N(0,1)`` drawn on the device (Philox4x32-10).
+    ``calls`` (a one-element int64 CUDA tensor): ``ldeq_sample_dev`` instead, which increments the counter on the device and
+    draws at offset ``calls << 32`` (``offset`` is ignored) -- what a CUDA graph replays with new noise every time."""
     h = _cabi.handle(mu.device.index or 0)
     mu = mu.contiguous().float()
     logvar = logvar.contiguous().float()
     z = torch.empty_like(mu)
     eps = torch.empty_like(mu) if want_eps else None
     with torch.cuda.device(mu.device):
-        h.check(h._lib.ldeq_sample(h.ptr, _p(mu), _p(logvar), _p(z), _p(eps), mu.numel(), C.c_uint64(seed & (2**64 - 1)),
-                                   C.c_uint64(offset & (2**64 - 1)), _stream()))
+        if calls is not None:
+            h.check(h._lib.ldeq_sample_dev(h.ptr, _p(mu), _p(logvar), _p(z), _p(eps), mu.numel(), C.c_uint64(seed & (2**64 - 1)),
+                                           _p(calls), _stream()))
+        else:
+            h.check(h._lib.ldeq_sample(h.ptr, _p(mu), _p(logvar), _p(z), _p(eps), mu.numel(), C.c_uint64(seed & (2**64 - 1)),
+                                       C.c_uint64(offset & (2**64 - 1)), _stream()))
     return z, eps
 
 
 class _Sample(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, mu, logvar, seed, offset):
-        z, eps = sample_raw(mu, logvar, seed, offset)
+    def forward(ctx, mu, logvar, seed, offset, calls):
+        z, eps = sample_raw(mu, logvar, seed, offset, calls=calls)
         ctx.save_for_backward(eps, logvar)
         return z
 
     @staticmethod
     def backward(ctx, dz):
         eps, logvar = ctx.saved_tensors
-        return dz, dz * eps * torch.exp(logvar * 0.5) * 0.5, None, None
+        return dz, dz * eps * torch.exp(logvar * 0.5) * 0.5, None, None, None
 
 
-def sample_reparam(mu, logvar, seed: int, offset: int = 0):
-    """Differentiable reparameterised sample (reference ``src/models/GOKU.jl:155-173``)."""
-    return _Sample.apply(mu, logvar, int(seed), int(offset))
+def sample_reparam(mu, logvar, seed: int, offset: int = 0, calls: torch.Tensor | None = None):
+    """Differentiable reparameterised sample (reference ``src/models/GOKU.jl:155-173``); ``calls``: see ``sample_raw``."""
+    return _Sample.apply(mu, logvar, int(seed), int(offset), calls)
 
 
-def elbo_raw(x: torch.Tensor, xhat: torch.Tensor, mus, logvars, beta: float, want_grad: bool = True,
+def elbo_raw(x: torch.Tensor, xhat: torch.Tensor, mus, logvars, beta, want_grad: bool = True,
              grad_scale: float = 1.0, logits: bool = False):
     """``ldeq_elbo_fwd_bwd``: ``x, xhat`` are ``[T, B, P]``; ``mus/logvars`` lists of ``[B, d_h]`` heads.
     Returns ``(loss3 = [total, reconstruction, kl], dxhat, dmus, dlogvars)``.  ``logits=True``
     (``ldeq_elbo_logits_fwd_bwd``): ``xhat`` holds the pre-activations of a sigmoid output layer; the gradient returned in
-    ``dxhat``'s place is with respect to them."""
+    ``dxhat``'s place is with respect to them.  ``beta`` is a Python float, or a 0-d Float32 CUDA tensor that the kernels
+    read on the device (the ``_dev`` entry points: a CUDA graph replays it with its current value)."""
     h = _cabi.handle(x.device.index or 0)
     x = _aligned16(x.contiguous().float())
     xhat = _aligned16(xhat.contiguous().float())
@@ -501,8 +509,15 @@ def elbo_raw(x: torch.Tensor, xhat: torch.Tensor, mus, logvars, beta: float, wan
     dlv_a = PA(*[l.data_ptr() for l in dlvs]) if want_grad else None
     hd = (C.c_int32 * max(nh, 1))(*[m.shape[1] for m in mus])
     with torch.cuda.device(x.device):
-        fn = h._lib.ldeq_elbo_logits_fwd_bwd if logits else h._lib.ldeq_elbo_fwd_bwd
-        h.check(fn(h.ptr, _p(x), _p(xhat), mu_a, lv_a, hd, nh, C.c_float(beta), B, T, P,
+        if isinstance(beta, torch.Tensor):
+            if not (beta.is_cuda and beta.dtype == torch.float32 and beta.numel() == 1):
+                raise TypeError("elbo: a tensor beta must be one Float32 element on the CUDA device")
+            fn = h._lib.ldeq_elbo_logits_fwd_bwd_dev if logits else h._lib.ldeq_elbo_fwd_bwd_dev
+            beta_arg = _p(beta)
+        else:
+            fn = h._lib.ldeq_elbo_logits_fwd_bwd if logits else h._lib.ldeq_elbo_fwd_bwd
+            beta_arg = C.c_float(beta)
+        h.check(fn(h.ptr, _p(x), _p(xhat), mu_a, lv_a, hd, nh, beta_arg, B, T, P,
                    C.c_float(grad_scale), _p(loss), _p(dxhat), dmu_a, dlv_a, _stream()))
     return loss, dxhat, dmus, dlvs
 
@@ -529,16 +544,17 @@ class _Elbo(torch.autograd.Function):
         return (None, g * dxhat, None, None, None, None, None, *[g * r for r in rest])
 
 
-def elbo_loss(x, xhat, mu, logvar, beta: float, logits: bool = False, unit_cotangent: bool = False, grad_scale: float = 1.0):
+def elbo_loss(x, xhat, mu, logvar, beta, logits: bool = False, unit_cotangent: bool = False, grad_scale: float = 1.0):
     """``loss_batch``'s reduction (reference ``examples/pendulum_friction-less/model_train.jl:225-238``):
     ``sum(mean((x - xhat)^2, dims=(2,3))) + beta * vector_kl(mu, logvar)`` as one fused forward+gradient pass.
     ``logits=True``: ``xhat`` are the pre-activations of the reconstructor's sigmoid output layer (folded into the kernel).
     ``unit_cotangent=True``: the result is differentiated directly (``loss.backward()``), never scaled further; a constant
     factor on the gradients (the data-parallel ``B_local / B_global``) then goes in as ``grad_scale`` -- the kernel writes the
-    gradients already multiplied by it, the returned loss value stays unscaled."""
+    gradients already multiplied by it, the returned loss value stays unscaled.  ``beta``: a float or a 0-d CUDA tensor
+    (``elbo_raw``)."""
     mus = list(mu) if isinstance(mu, (tuple, list)) else [mu]
     lvs = list(logvar) if isinstance(logvar, (tuple, list)) else [logvar]
-    return _Elbo.apply(x, xhat, float(beta), len(mus), bool(logits), bool(unit_cotangent), float(grad_scale), *mus, *lvs)
+    return _Elbo.apply(x, xhat, beta if isinstance(beta, torch.Tensor) else float(beta), len(mus), bool(logits), bool(unit_cotangent), float(grad_scale), *mus, *lvs)
 
 
 def adamw_step(params: torch.Tensor, grads: torch.Tensor, m: torch.Tensor, v: torch.Tensor, step: int, lr=1e-3,
@@ -550,6 +566,32 @@ def adamw_step(params: torch.Tensor, grads: torch.Tensor, m: torch.Tensor, v: to
         h.check(h._lib.ldeq_adamw_step(h.ptr, _p(params), _p(grads), _p(m), _p(v), params.numel(), float(lr),
                                        float(betas[0]), float(betas[1]), float(eps), C.c_float(decay), int(step),
                                        C.c_float(grad_scale), _stream()))
+
+
+def adamw_step_dev(params: torch.Tensor, grads: torch.Tensor, m: torch.Tensor, v: torch.Tensor, state: torch.Tensor, lr=1e-3,
+                   betas=(0.9, 0.999), eps=1e-8, decay=1e-3, grad_scale: float = 1.0):
+    """``ldeq_adamw_step_dev``: ``adamw_step`` with the step count and the beta powers in ``state``, a 3-element Float64 CUDA
+    tensor holding ``ldeq_adamw_state`` (``int64 step`` bit-cast, ``beta1^step``, ``beta2^step``), advanced on the device."""
+    h = _cabi.handle(params.device.index or 0)
+    assert params.is_contiguous() and grads.is_contiguous() and m.is_contiguous() and v.is_contiguous()
+    if not (state.is_cuda and state.dtype == torch.float64 and state.numel() == 3 and state.is_contiguous()):
+        raise TypeError("adamw_step_dev: state must be a contiguous 3-element Float64 CUDA tensor (ldeq_adamw_state)")
+    with torch.cuda.device(params.device):
+        h.check(h._lib.ldeq_adamw_step_dev(h.ptr, _p(params), _p(grads), _p(m), _p(v), params.numel(), float(lr),
+                                           float(betas[0]), float(betas[1]), float(eps), C.c_float(decay), _p(state),
+                                           C.c_float(grad_scale), _stream()))
+
+
+def adamw_state(step: int, betas=(0.9, 0.999), device=None) -> torch.Tensor:
+    """The ``ldeq_adamw_state`` after ``step`` steps, as ``adamw_step_dev`` keeps it: the beta powers are the running Float64
+    products of ``ldeq_adamw_step`` (Python floats are IEEE doubles: same multiplications, same bits)."""
+    p1 = p2 = 1.0
+    for _ in range(step):
+        p1 *= float(betas[0])
+        p2 *= float(betas[1])
+    st = torch.tensor([0.0, p1, p2], dtype=torch.float64)
+    st.view(torch.int64)[0] = int(step)
+    return st.to(device) if device is not None else st
 
 
 def allreduce_adamw_step(params, peer_grad_ptrs, m, v, step: int, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, decay=1e-3,

@@ -11,7 +11,9 @@ from __future__ import annotations
 import torch
 import torch.distributed as dist
 
-from .solve import adamw_step, allreduce_adamw_step, elbo_loss
+from . import _cabi
+from . import model as _model
+from .solve import _tgrid, adamw_state, adamw_step, adamw_step_dev, allreduce_adamw_step, elbo_loss
 
 
 def loss_batch(model, x, t, beta, variational, fused_output: bool = True, unit_cotangent: bool = False, grad_scale: float = 1.0):
@@ -97,6 +99,12 @@ class ADAMW:
         else:
             raise RuntimeError("the optimiser step runs in libldeq.so on a CUDA device (no CPU fallback)")
 
+    def step_dev(self, state: torch.Tensor, grad_scale: float = 1.0):
+        """``step`` with the step count and the beta powers in the device tensor ``state`` (``adamw_step_dev``), which the
+        kernel advances; ``step_count`` is left to the caller (``GraphedTrainStep`` keeps it as the host mirror)."""
+        f = self.flat
+        adamw_step_dev(f.flat, f.grad, f.m, f.v, state, self.eta, self.beta, self.eps, self.decay, grad_scale)
+
     def fused_allreduce_step(self, grad_scale: float = 1.0):
         """All-reduce + AdamW in ONE kernel over NVLink peer memory (needs ``FlatParams(..., symmetric=True)``):
         barrier (all buckets written) -> sum in rank order + AdamW -> barrier (every rank has read every bucket / written
@@ -148,3 +156,91 @@ def train_step(model, flat: FlatParams, opt: ADAMW, x_local, t, beta, variationa
         opt.step()
     mark("update")
     return loss.detach()
+
+
+class GraphedTrainStep:
+    """``train_step`` captured once as a CUDA graph and replayed: ``loss = step(x, beta)``.
+
+    At the reference's batch of 64 every kernel of a step runs for microseconds and the eager step is bound by launches and
+    host work; a replay is one launch.  The per-step values live in device memory: the AdamW step state, the sample counter
+    (``ldeq_sample_dev``) and beta (the ELBO's ``_dev`` entry points), so replay k computes what eager step k computes, bit
+    for bit.  ``opt.step_count`` and the module's sample counter stay the host mirrors: each call advances them, and eager
+    calls in between (a validation ``loss_batch``) keep working on the same handle and stream; when the mirrors moved
+    without the graph (an eager ``train_step``), the device state is refreshed from them before the replay.
+
+    Built for single-GPU GOKU training on its default path: Pendulum / Pendulum_friction / NVRTC right-hand sides with
+    ``ForwardDiffSensitivity()``, the pattern-extractor kernels, the fused logits ELBO and AdamW.  Everything else is refused
+    before any capture: LatentODE (its reverse passes need the host), ``DiscreteAdjoint()``, world size > 1 and a
+    reconstructor without the sigmoid output layer the fused loss needs.  ``x`` must keep ``x_example``'s shape, ``t`` is
+    fixed, and the noise seed is ``torch.initial_seed()`` at construction.  Construction warms the exact shapes up on a side
+    stream (modules, the device grid, the workspaces) and leaves parameters, gradients, ``m``, ``v``, ``opt.step_count`` and
+    the sample counter as it found them."""
+
+    def __init__(self, model, flat: FlatParams, opt: ADAMW, x_example: torch.Tensor, t, variational: bool = True, warmup: int = 2):
+        if not x_example.is_cuda:
+            raise RuntimeError("GraphedTrainStep: the batch must be a CUDA tensor")
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            raise NotImplementedError("GraphedTrainStep: single GPU only (the gradient all-reduce is not captured)")
+        if flat.symm is not None:
+            raise NotImplementedError("GraphedTrainStep: FlatParams(symmetric=True) belongs to the fused multi-GPU step")
+        if not isinstance(model.model_type, _model.GOKU):
+            raise NotImplementedError("GraphedTrainStep: GOKU models only; LatentODE's reverse passes need the host (the MLP tape "
+                                      "check and the continuous adjoint)")
+        diffeq = model.decoder.diffeq
+        opts = _model._opts_from_kwargs(diffeq.kwargs, getattr(diffeq, "sensealg", None), getattr(diffeq, "solver", None))
+        if opts.sensealg != _cabi.SENSE_FORWARD_DUAL:
+            raise NotImplementedError("GraphedTrainStep: ForwardDiffSensitivity() only; the discrete adjoint checks its tape on the host")
+        if _model._logits_layers(model.decoder) is None:
+            raise NotImplementedError("GraphedTrainStep: the reconstructor must end in a Dense layer with the sigmoid output "
+                                      "activation (the fused logits ELBO)")
+        self.model, self.flat, self.opt, self.variational = model, flat, opt, variational
+        dev = x_example.device
+        self._t = _tgrid(t)
+        self._x = x_example.detach().clone(memory_format=torch.contiguous_format)
+        self._beta = torch.zeros((), dtype=torch.float32, device=dev)
+        self._state = torch.zeros(3, dtype=torch.float64, device=dev)   # ldeq_adamw_state
+        self._calls = torch.zeros(1, dtype=torch.int64, device=dev)
+        saved = [b.clone() for b in (flat.flat, flat.grad, flat.m, flat.v)]
+        step0, calls0 = opt.step_count, _model._sample_calls
+        cur = torch.cuda.current_stream(dev)
+        side = torch.cuda.Stream(dev)
+        side.wait_stream(cur)
+        with torch.cuda.stream(side):
+            for _ in range(warmup):
+                self._body()
+        cur.wait_stream(side)
+        for b, v in zip((flat.flat, flat.grad, flat.m, flat.v), saved):
+            b.copy_(v)
+        opt.step_count = step0
+        _model._sample_calls = calls0
+        self._graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self._graph):
+            self._loss = self._body()
+        self._draws = _model._sample_calls - calls0   # samples per step
+        _model._sample_calls = calls0
+        self._synced = None   # (step_count, sample counter) the device state holds
+
+    def _body(self):
+        self.flat.zero_grad()
+        with _model.device_sample_counter(self._calls):
+            loss = loss_batch(self.model, self._x, self._t, self._beta, self.variational, unit_cotangent=True)
+        loss.backward()
+        self.opt.step_dev(self._state)
+        return loss.detach()
+
+    def __call__(self, x: torch.Tensor, beta) -> torch.Tensor:
+        """One training step on ``x`` (``x_example``'s shape) with KL weight ``beta`` (float or 0-d CUDA tensor); returns the
+        loss as a device tensor, without synchronising."""
+        if (self.opt.step_count, _model._sample_calls) != self._synced:
+            self._state.copy_(adamw_state(self.opt.step_count, self.opt.beta))
+            self._calls.fill_(_model._sample_calls)
+        self._x.copy_(x)
+        if isinstance(beta, torch.Tensor):
+            self._beta.copy_(beta)
+        else:
+            self._beta.fill_(beta)
+        self._graph.replay()
+        self.opt.step_count += 1
+        _model._sample_calls += self._draws
+        self._synced = (self.opt.step_count, _model._sample_calls)
+        return self._loss.clone()
