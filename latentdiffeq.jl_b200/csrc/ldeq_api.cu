@@ -8,16 +8,11 @@
 #include <cstring>
 
 #include "ldeq_internal.h"
-#include "ldeq_rhs.cuh"
 #include "ldeq_tsit5.cuh"
+#include "ldeq_fwdsens.cuh"
 #include "ldeq_julia_trig.cuh"
 
 namespace ldeq {
-
-// ldeq_erk.cu: the forward kernel for solver = DP5 / BS3 / RK4 (built-in right-hand sides)
-cudaError_t launch_erk_fwd(int solver, int dtype, bool friction, bool with_tape, const void* z0, const void* theta, const double* tg, int B,
-                           int T, const KOpts& ko, void* traj, int32_t* ret, int32_t* na, int32_t* nr, const TapeView<float>& tv,
-                           const GridInfo& gi, cudaStream_t s);
 
 int set_err(ldeq_handle* h, int code, const char* what, cudaError_t ce) {
     if (h) {
@@ -135,88 +130,66 @@ KOpts to_kopts(const ldeq_opts* o) {
     return k;
 }
 
-// The forward kernel fills the tape's own copies (theta, grid, statistics) itself; a replay into a fresh tape (tape_heal)
-// reads theta / the grid FROM the tape, where they already are.
-template <class S>
-static TapeView<S> fwd_tape_view(const ldeq_tape* tape, const void* theta, const double* tg) {
-    return TapeView<S>{tape->t, (S*)tape->u, tape->info, tape->cap,
-                       theta == tape->theta ? nullptr : (S*)tape->theta, tg == tape->tgrid ? nullptr : tape->tgrid,
-                       tape->retcode, tape->naccept, tape->nreject};
-}
-
-template <class S, bool FRICTION, bool TAPE>
-static cudaError_t launch_fwd(const void* z0, const void* theta, const double* tg, int B, int T, const KOpts& ko,
-                              void* traj, int32_t* ret, int32_t* na, int32_t* nr, const ldeq_tape* tape,
-                              const GridInfo& gi, cudaStream_t s) {
-    TapeView<S> tv{nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr};
-    if (TAPE) tv = fwd_tape_view<S>(tape, theta, tg);
-    const int grid = (B + LDEQ_FWD_THREADS - 1) / LDEQ_FWD_THREADS;
-    const size_t smem = Ring<S, 2>::bytes(LDEQ_FWD_THREADS) + (T <= LDEQ_TGRID_SMEM_MAX ? (size_t)T * sizeof(double) : 0);
-    tsit5_fwd_kernel<PendulumRHS<S, FRICTION>, S, TAPE><<<grid, LDEQ_FWD_THREADS, smem, s>>>(
-        (const S*)z0, (const S*)theta, tg, B, T, ko, (S*)traj, ret, na, nr, tv, gi);
-    return cudaGetLastError();
-}
-
-// The discrete-adjoint kernels re-deal the trajectories of a CTA to lanes by their accepted-step count (measured at
-// 2^20 x 200: 1.135 -> 1.095 ms); LDEQ_BWD_SORT=0 keeps the batch order (A/B switch; the results are identical bit for bit).
-int bwd_sort_lanes() {
-    static const int on = [] { const char* e = getenv("LDEQ_BWD_SORT"); return (e && e[0] == '0') ? 0 : 1; }();
-    return on;
-}
-
-template <class S, bool FRICTION>
-static cudaError_t launch_bwd(const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    TapeView<S> tv{tape->t, (S*)tape->u, tape->info, tape->cap, nullptr, nullptr, nullptr, nullptr, nullptr};
-    const int grid = (tape->B + LDEQ_BWD_THREADS - 1) / LDEQ_BWD_THREADS;
-    const size_t smem =
-        Ring<S, 2>::bytes(LDEQ_BWD_THREADS) + (tape->T <= LDEQ_TGRID_SMEM_MAX ? (size_t)tape->T * sizeof(double) : 0);
-    tsit5_bwd_kernel<PendulumRHS<S, FRICTION>, S><<<grid, LDEQ_BWD_THREADS, smem, s>>>(
-        (const S*)tape->theta, tape->tgrid, tape->B, tape->T, (const S*)dtraj, tv, tape->retcode, tape->naccept,
-        (S*)dz0, (S*)dtheta, GridInfo{tape->grid_t0, tape->grid_h, tape->grid_uniform, ld, bwd_sort_lanes()});
-    return cudaGetLastError();
-}
-
 static size_t align_up(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// shared memory of one CTA for a state of z_dim elements of `es` bytes: per-lane ring + staged time grid
+// ---- the three passes of a GOKU solve: one launch of an entry of the kernel table, for every right-hand side ----------
+// shared memory of one CTA for a state of z_dim elements of `es` bytes: per-lane ring (Ring<S, ZD>) + staged time grid
 static size_t ring_smem(int z_dim, size_t es, int threads, int T) {
     int rows = LDEQ_RING_BYTES / (z_dim * (int)es);
     rows = rows >= 64 ? 64 : rows >= 32 ? 32 : rows >= 16 ? 16 : rows >= 8 ? 8 : 4;
     return (size_t)rows * threads * z_dim * es + (T <= LDEQ_TGRID_SMEM_MAX ? (size_t)T * sizeof(double) : 0);
 }
 
-// kernels of an NVRTC-compiled user right-hand side (ldeq_user_rhs.cu): fn[] = {fwd f32, fwd f32 tape, fwd f64,
-// fwd f64 tape, bwd f32, bwd f64}; same signatures as the built-in instantiations
-static cudaError_t launch_user_fwd(void* const* fn, const ldeq_rhs* rhs, int dtype, const void* z0, const void* theta, const double* tg,
-                                   int B, int T, const KOpts& ko, void* traj, int32_t* ret, int32_t* na, int32_t* nr,
-                                   const ldeq_tape* tape, const GridInfo& gi, cudaStream_t s) {
-    TapeView<float> tv{nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr};  // identical layout for float and double
-    if (tape) tv = fwd_tape_view<float>(tape, theta, tg);
+// The step records of a tape as the kernels see them.  TapeView<float> and TapeView<double> have the same layout (pointers
+// + one int): the float form is passed for both.
+static TapeView<float> tape_view(const ldeq_tape* tape) {
+    return TapeView<float>{tape->t, (float*)tape->u, tape->info, tape->cap, nullptr, nullptr, nullptr, nullptr, nullptr};
+}
+
+// Forward solve.  With a tape the kernel fills the tape's own copies (theta, grid, statistics) itself; a replay into a
+// fresh tape (tape_heal) reads theta / the grid FROM the tape, where they already are.
+static cudaError_t launch_fwd(const GokuKernels& k, int z_dim, int dtype, const void* z0, const void* theta, const double* tg,
+                              int B, int T, const KOpts& ko, void* traj, int32_t* ret, int32_t* na, int32_t* nr,
+                              const ldeq_tape* tape, const GridInfo& gi, cudaStream_t s) {
+    TapeView<float> tv{};
+    if (tape) {
+        tv = tape_view(tape);
+        tv.theta = theta == tape->theta ? nullptr : (float*)tape->theta;
+        tv.tgrid = tg == tape->tgrid ? nullptr : tape->tgrid;
+        tv.ret = tape->retcode;
+        tv.na = tape->naccept;
+        tv.nr = tape->nreject;
+    }
     KOpts kov = ko;
     GridInfo giv = gi;
     void* args[] = {&z0, &theta, &tg, &B, &T, &kov, &traj, &ret, &na, &nr, &tv, &giv};
     const int grid = (B + LDEQ_FWD_THREADS - 1) / LDEQ_FWD_THREADS;
     const size_t es = dtype == LDEQ_F32 ? 4 : 8;
-    void* kfn = fn[(dtype == LDEQ_F32 ? 0 : 2) + (tape ? 1 : 0)];
-    return cudaLaunchKernel(kfn, dim3(grid), dim3(LDEQ_FWD_THREADS), args, ring_smem(rhs->z_dim, es, LDEQ_FWD_THREADS, T), s);
+    return cudaLaunchKernel(k.fwd[dtype][tape ? 1 : 0], dim3(grid), dim3(LDEQ_FWD_THREADS), args,
+                            ring_smem(z_dim, es, LDEQ_FWD_THREADS, T), s);
 }
-static cudaError_t launch_user_bwd(void* const* fn, const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    TapeView<float> tv{tape->t, (float*)tape->u, tape->info, tape->cap, nullptr, nullptr, nullptr, nullptr, nullptr};
+
+// Discrete adjoint of the taped steps.  The kernel re-deals the trajectories of a CTA to lanes by their accepted-step count
+// (GridInfo::sort; measured at 2^20 x 200: 1.135 -> 1.095 ms, the results are identical bit for bit).
+static cudaError_t launch_bwd(const GokuKernels& k, const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta,
+                              cudaStream_t s) {
+    TapeView<float> tv = tape_view(tape);
     const void* theta = tape->theta;
     const double* tg = tape->tgrid;
     int B = tape->B, T = tape->T;
     const int32_t* ret = tape->retcode;
     const int32_t* na = tape->naccept;
-    GridInfo giv{tape->grid_t0, tape->grid_h, tape->grid_uniform, ld, bwd_sort_lanes()};
-    void* args[] = {&theta, &tg, &B, &T, &dtraj, &tv, &ret, &na, &dz0, &dtheta, &giv};
+    GridInfo gi{tape->grid_t0, tape->grid_h, tape->grid_uniform, ld, 1};
+    void* args[] = {&theta, &tg, &B, &T, &dtraj, &tv, &ret, &na, &dz0, &dtheta, &gi};
     const int grid = (B + LDEQ_BWD_THREADS - 1) / LDEQ_BWD_THREADS;
     const size_t es = tape->dtype == LDEQ_F32 ? 4 : 8;
-    void* kfn = fn[tape->dtype == LDEQ_F32 ? 4 : 5];
-    return cudaLaunchKernel(kfn, dim3(grid), dim3(LDEQ_BWD_THREADS), args, ring_smem(tape->z_dim, es, LDEQ_BWD_THREADS, T), s);
+    return cudaLaunchKernel(k.bwd[tape->dtype], dim3(grid), dim3(LDEQ_BWD_THREADS), args, ring_smem(tape->z_dim, es, LDEQ_BWD_THREADS, T), s);
 }
 
-// fn[6..9] = forward-dual pullback {theta-seeded f32, u0-seeded f32, theta-seeded f64, u0-seeded f64}
-static cudaError_t launch_user_fwdsens(void* const* fn, const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
+// Forward-dual pullback: the theta-seeded and the u0-seeded dual re-solve.  Lanes are re-dealt by the primal step count
+// (sort_key = naccept, ldeq_fwdsens.cuh).
+static cudaError_t launch_fwdsens(const GokuKernels& k, const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta,
+                                  cudaStream_t s) {
     const void* z0 = tape->u;
     const void* theta = tape->theta;
     const double* tg = tape->tgrid;
@@ -224,14 +197,13 @@ static cudaError_t launch_user_fwdsens(void* const* fn, const ldeq_tape* tape, c
     GridInfo gi{tape->grid_t0, tape->grid_h, tape->grid_uniform, ld};
     KOpts kov = tape->kopts;
     const int32_t* ret = tape->retcode;
-    const int32_t* key = tape->naccept;  // lanes re-dealt by the primal step count (ldeq_fwdsens.cuh)
-    const int grid = (B + 127) / 128;
-    const int base = tape->dtype == LDEQ_F32 ? 6 : 8;
+    const int32_t* key = tape->naccept;
+    const int grid = (B + LDEQ_FWDSENS_THREADS - 1) / LDEQ_FWDSENS_THREADS;
     void* args_p[] = {&z0, &theta, &tg, &B, &gi, &T, &kov, &np, &key, &dtraj, &ret, &dtheta};
-    cudaError_t e = cudaLaunchKernel(fn[base], dim3(grid), dim3(128), args_p, 0, s);
+    cudaError_t e = cudaLaunchKernel(k.fwdsens[tape->dtype][0], dim3(grid), dim3(LDEQ_FWDSENS_THREADS), args_p, 0, s);
     if (e != cudaSuccess) return e;
     void* args_u[] = {&z0, &theta, &tg, &B, &gi, &T, &kov, &np, &key, &dtraj, &ret, &dz0};
-    return cudaLaunchKernel(fn[base + 1], dim3(grid), dim3(128), args_u, 0, s);
+    return cudaLaunchKernel(k.fwdsens[tape->dtype][1], dim3(grid), dim3(LDEQ_FWDSENS_THREADS), args_u, 0, s);
 }
 
 // Pinned two-int mirrors + events come from a per-handle pool: cudaMallocHost / cudaFreeHost cost milliseconds of host time
@@ -299,33 +271,10 @@ static int tape_alloc(ldeq_handle* h, ldeq_tape* tape, int cap, cudaStream_t s) 
     return LDEQ_OK;
 }
 
-static cudaError_t dispatch_fwd(ldeq_handle* h, int solver, const ldeq_rhs* rhs, int dtype, const void* z0, const void* theta,
-                                const double* tg, int B, int T, const KOpts& ko, void* traj, int32_t* ret, int32_t* na, int32_t* nr,
-                                const ldeq_tape* tape, const GridInfo& gi, cudaStream_t s) {
-    if (rhs->kind < 0) {
-        void* const* fn = user_rhs_kernels(h, rhs, solver);
-        if (!fn) return cudaErrorLaunchFailure;  // h->err holds the NVRTC log
-        return launch_user_fwd(fn, rhs, dtype, z0, theta, tg, B, T, ko, traj, ret, na, nr, tape, gi, s);
-    }
-    const bool friction = rhs->kind == LDEQ_RHS_PENDULUM_FRICTION;
-    if (solver != LDEQ_SOLVER_TSIT5) {
-        TapeView<float> tv{nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr};
-        if (tape) tv = fwd_tape_view<float>(tape, theta, tg);
-        return launch_erk_fwd(solver, dtype, friction, tape != nullptr, z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s);
-    }
-#define LDEQ_DISPATCH_FWD(S)                                                                              \
-    (tape ? (friction ? launch_fwd<S, true, true>(z0, theta, tg, B, T, ko, traj, ret, na, nr, tape, gi, s)    \
-                      : launch_fwd<S, false, true>(z0, theta, tg, B, T, ko, traj, ret, na, nr, tape, gi, s))  \
-          : (friction ? launch_fwd<S, true, false>(z0, theta, tg, B, T, ko, traj, ret, na, nr, tape, gi, s)   \
-                      : launch_fwd<S, false, false>(z0, theta, tg, B, T, ko, traj, ret, na, nr, tape, gi, s)))
-    return dtype == LDEQ_F32 ? LDEQ_DISPATCH_FWD(float) : LDEQ_DISPATCH_FWD(double);
-#undef LDEQ_DISPATCH_FWD
-}
-
 // A tape whose capacity turned out too small heals itself before the backward pass: the forward
 // solve is replayed (same inputs, same arithmetic, hence the same steps) into a tape sized by the
 // largest accepted-step count the first pass reported.  Costs one extra forward kernel, only then.
-static int tape_heal(ldeq_handle* h, ldeq_tape* tape, cudaStream_t s) {
+static int tape_heal(ldeq_handle* h, const GokuKernels& k, ldeq_tape* tape, cudaStream_t s) {
     if (tape->checked) return LDEQ_OK;
     LDEQ_CUDA(cudaEventSynchronize(tape->ready));
     tape->checked = true;
@@ -338,12 +287,11 @@ static int tape_heal(ldeq_handle* h, ldeq_tape* tape, cudaStream_t s) {
     cudaMemcpyAsync(tape->theta, old.theta, (size_t)tape->B * tape->p_dim * es, cudaMemcpyDeviceToDevice, s);
     cudaMemcpyAsync(tape->tgrid, old.tgrid, (size_t)tape->T * 8, cudaMemcpyDeviceToDevice, s);
     // step 0 of the old tape holds u0 for every trajectory (capacity is always >= 1)
-    cudaError_t e = dispatch_fwd(h, tape->solver, tape->rhs, tape->dtype, old.u, tape->theta,
-                                 tape->tgrid, tape->B, tape->T, tape->kopts, nullptr, nullptr, nullptr,
-                                 nullptr, tape, GridInfo{tape->grid_t0, tape->grid_h, tape->grid_uniform, tape->B}, s);
+    cudaError_t e = launch_fwd(k, tape->z_dim, tape->dtype, old.u, tape->theta, tape->tgrid, tape->B, tape->T, tape->kopts, nullptr,
+                               nullptr, nullptr, nullptr, tape, GridInfo{tape->grid_t0, tape->grid_h, tape->grid_uniform, tape->B}, s);
     h->launches += 1;
     cudaFreeAsync(old.base, s);
-    if (e != cudaSuccess) return set_err(h, LDEQ_ERR_CUDA, "tsit5_fwd_kernel (tape replay) launch", e);
+    if (e != cudaSuccess) return set_err(h, LDEQ_ERR_CUDA, "forward solve (tape replay) launch", e);
     return LDEQ_OK;
 }
 
@@ -431,9 +379,11 @@ int ldeq_rhs_builtin(ldeq_handle* h, int kind, ldeq_rhs** out) {
     if (kind != LDEQ_RHS_PENDULUM && kind != LDEQ_RHS_PENDULUM_FRICTION)
         return set_err(h, LDEQ_ERR_INVALID, "unknown built-in rhs kind");
     ldeq_rhs* r = new ldeq_rhs();
-    r->kind = kind;
     r->z_dim = 2;
     r->p_dim = 1;
+    builtin_solve_kernels(kind, r->kernels);
+    builtin_fwdsens_tsit5(kind, r->kernels);
+    builtin_fwdsens_erk(kind, r->kernels);
     *out = r;
     return LDEQ_OK;
 }
@@ -469,10 +419,12 @@ static int solve_fwd_slab(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const 
     const bool fwd_dual = tape_out && opts->sensealg == LDEQ_SENSE_FORWARD_DUAL;
     ldeq_tape* tape = nullptr;
     int rc;
+    if (tape_out) *tape_out = nullptr;
+    const GokuKernels* k = rhs_kernels(h, rhs, opts->solver);
+    if (!k) return LDEQ_ERR_COMPILE;  // h->err holds the NVRTC log
     if (tape_out) {
-        *tape_out = nullptr;
         tape = new ldeq_tape();
-        tape->dtype = dtype; tape->rhs_kind = rhs->kind; tape->rhs = rhs; tape->B = B; tape->T = T;
+        tape->dtype = dtype; tape->rhs = rhs; tape->B = B; tape->T = T;
         tape->z_dim = ZD; tape->p_dim = PD; tape->kopts = ko;
         tape->grid_t0 = grid.t0; tape->grid_h = grid.h; tape->grid_uniform = grid.uniform;
         long long cap = opts->tape_steps;
@@ -500,8 +452,8 @@ static int solve_fwd_slab(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const 
         }
         // theta, the grid, the statistics and u0 (record 0) reach the tape through the forward kernel itself (TapeView)
     }
-    cudaError_t e = dispatch_fwd(h, opts->solver, rhs, dtype, z0, theta, grid.d, B, T, ko, traj_out, retcode, naccept, nreject, tape,
-                                 GridInfo{grid.t0, grid.h, grid.uniform, ld}, s);
+    cudaError_t e = launch_fwd(*k, ZD, dtype, z0, theta, grid.d, B, T, ko, traj_out, retcode, naccept, nreject, tape,
+                               GridInfo{grid.t0, grid.h, grid.uniform, ld}, s);
     h->launches += 1;
     if (e != cudaSuccess) {
         if (tape) {
@@ -510,8 +462,7 @@ static int solve_fwd_slab(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const 
             slot_put(h, tape, s);
             delete tape;
         }
-        if (rhs->kind < 0 && e == cudaErrorLaunchFailure && !h->err.empty() && h->err.compare(0, 5, "NVRTC") == 0) return LDEQ_ERR_COMPILE;
-        return set_err(h, LDEQ_ERR_CUDA, "tsit5_fwd_kernel launch", e);
+        return set_err(h, LDEQ_ERR_CUDA, "forward solve launch", e);
     }
     if (tape) {
         if (tape->ready) {
@@ -525,29 +476,19 @@ static int solve_fwd_slab(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const 
 
 // reverse pass of one slab (a single-part tape); dtraj / dz0 / dtheta already offset, ld = row stride of dtraj
 static int solve_bwd_slab(ldeq_handle* h, ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    void* const* ufn = nullptr;
-    if (tape->rhs_kind < 0 && !(ufn = user_rhs_kernels(h, tape->rhs, tape->solver))) return LDEQ_ERR_COMPILE;
+    const GokuKernels* k = rhs_kernels(h, tape->rhs, tape->solver);
+    if (!k) return LDEQ_ERR_COMPILE;
     if (tape->sense == LDEQ_SENSE_FORWARD_DUAL) {
-        const cudaError_t e2 = tape->rhs_kind < 0 ? launch_user_fwdsens(ufn, tape, dtraj, ld, dz0, dtheta, s)
-                                                  : launch_fwdsens(tape, dtraj, ld, dz0, dtheta, s);
+        const cudaError_t e = launch_fwdsens(*k, tape, dtraj, ld, dz0, dtheta, s);
         h->launches += 2;
-        if (e2 != cudaSuccess) return set_err(h, LDEQ_ERR_CUDA, "tsit5_fwdsens_kernel launch", e2);
+        if (e != cudaSuccess) return set_err(h, LDEQ_ERR_CUDA, "forward-dual pullback launch", e);
         return LDEQ_OK;
     }
-    int rc = tape_heal(h, tape, s);
+    int rc = tape_heal(h, *k, tape, s);
     if (rc) return rc;
-    const bool fr = tape->rhs_kind == LDEQ_RHS_PENDULUM_FRICTION;
-    cudaError_t e;
-    if (tape->rhs_kind < 0)
-        e = launch_user_bwd(ufn, tape, dtraj, ld, dz0, dtheta, s);
-    else if (tape->solver != LDEQ_SOLVER_TSIT5)
-        e = launch_erk_bwd(tape, dtraj, ld, dz0, dtheta, s);
-    else if (tape->dtype == LDEQ_F32)
-        e = fr ? launch_bwd<float, true>(tape, dtraj, ld, dz0, dtheta, s) : launch_bwd<float, false>(tape, dtraj, ld, dz0, dtheta, s);
-    else
-        e = fr ? launch_bwd<double, true>(tape, dtraj, ld, dz0, dtheta, s) : launch_bwd<double, false>(tape, dtraj, ld, dz0, dtheta, s);
+    const cudaError_t e = launch_bwd(*k, tape, dtraj, ld, dz0, dtheta, s);
     h->launches += 1;
-    if (e != cudaSuccess) return set_err(h, LDEQ_ERR_CUDA, "tsit5_bwd_kernel launch", e);
+    if (e != cudaSuccess) return set_err(h, LDEQ_ERR_CUDA, "discrete adjoint launch", e);
     return LDEQ_OK;
 }
 
@@ -653,7 +594,7 @@ int ldeq_solve_fwd(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const void* z
     if (tape_out && opts->sensealg != LDEQ_SENSE_FORWARD_DUAL)
         return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_fwd: a discrete-adjoint tape is not available under CUDA graph capture (its "
                                                 "reverse pass reads the tape's overflow count on the host)");
-    if (rhs->kind < 0 && opts->solver != LDEQ_SOLVER_TSIT5 && !rhs->alt[opts->solver].module)
+    if (!rhs->built(opts->solver))
         return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_fwd: the right-hand side has not been compiled for this solver yet, and NVRTC "
                                                 "cannot run under CUDA graph capture: solve once outside the capture first");
     ldeq_handle::GridEntry* g = nullptr;
@@ -676,7 +617,7 @@ int ldeq_solve_bwd(ldeq_handle* h, ldeq_tape* tape, const void* dtraj, void* dz0
         if (!tape->parts.empty() || tape->sense != LDEQ_SENSE_FORWARD_DUAL)
             return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_bwd: only the forward-dual pullback of a device solve is available under CUDA "
                                                     "graph capture (the discrete adjoint reads the tape's overflow count on the host)");
-        if (tape->rhs_kind < 0 && tape->solver != LDEQ_SOLVER_TSIT5 && !tape->rhs->alt[tape->solver].module)
+        if (!tape->rhs->built(tape->solver))
             return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_bwd: the right-hand side has not been compiled for this solver yet, and "
                                                     "NVRTC cannot run under CUDA graph capture");
     }
@@ -743,7 +684,7 @@ int ldeq_solve_fwd_host(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const vo
     ldeq_tape* parent = nullptr;
     if (tape_out) {
         parent = new ldeq_tape();
-        parent->dtype = dtype; parent->rhs_kind = rhs->kind; parent->rhs = rhs; parent->B = B; parent->T = T;
+        parent->dtype = dtype; parent->rhs = rhs; parent->B = B; parent->T = T;
         parent->z_dim = rhs->z_dim; parent->p_dim = rhs->p_dim; parent->sense = opts->sensealg; parent->solver = opts->solver;
     }
     const int ns = slab_count(B);

@@ -1,79 +1,35 @@
-// ldeq_erk.cu -- the GOKU integrator kernels (ldeq_tsit5.cuh) instantiated with the table-driven methods of
-// ldeq_erk.cuh: the diffeq struct's `solver` field set to DP5(), BS3() or RK4() (SURVEY.md 8(f)4; the reference's own
-// structs use Tsit5(), pendulum.jl:11,58).  Same thread-per-trajectory kernels, ring, tape and discrete adjoint.
+// ldeq_erk.cu -- the forward and discrete-adjoint kernels of the built-in right-hand sides (ldeq_tsit5.cuh), one set per
+// value of the diffeq struct's `solver` field: Tsit5 (the reference's structs, pendulum.jl:11,58) and the table-driven
+// methods of ldeq_erk.cuh, DP5(), BS3() and RK4() (SURVEY.md 8(f)4).  Same thread-per-trajectory kernels, ring, tape and
+// discrete adjoint.
 #include "ldeq_internal.h"
 #include "ldeq_rhs.cuh"
 #include "ldeq_tsit5.cuh"
 
 namespace ldeq {
 
-template <class M, class S, bool FRICTION, bool TAPE>
-static cudaError_t fwd_t(const void* z0, const void* theta, const double* tg, int B, int T, const KOpts& ko, void* traj, int32_t* ret,
-                         int32_t* na, int32_t* nr, const TapeView<S>& tv, const GridInfo& gi, cudaStream_t s) {
-    const int grid = (B + LDEQ_FWD_THREADS - 1) / LDEQ_FWD_THREADS;
-    const size_t smem = Ring<S, 2>::bytes(LDEQ_FWD_THREADS) + (T <= LDEQ_TGRID_SMEM_MAX ? (size_t)T * sizeof(double) : 0);
-    erk_fwd_kernel<M, PendulumRHS<S, FRICTION>, S, TAPE><<<grid, LDEQ_FWD_THREADS, smem, s>>>(
-        (const S*)z0, (const S*)theta, tg, B, T, ko, (S*)traj, ret, na, nr, tv, gi);
-    return cudaGetLastError();
-}
-
-template <class M, class S>
-static cudaError_t fwd_s(bool friction, bool with_tape, const void* z0, const void* theta, const double* tg, int B, int T, const KOpts& ko,
-                         void* traj, int32_t* ret, int32_t* na, int32_t* nr, const TapeView<float>& tvf, const GridInfo& gi, cudaStream_t s) {
-    // TapeView<float> and TapeView<double> have the same layout (pointers + one int); the caller fills the float form
-    TapeView<S> tv{tvf.t, (S*)tvf.u, tvf.info, tvf.cap, (S*)tvf.theta, tvf.tgrid, tvf.ret, tvf.na, tvf.nr};
-    if (with_tape)
-        return friction ? fwd_t<M, S, true, true>(z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s)
-                        : fwd_t<M, S, false, true>(z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s);
-    return friction ? fwd_t<M, S, true, false>(z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s)
-                    : fwd_t<M, S, false, false>(z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s);
-}
-
-template <class M>
-static cudaError_t fwd_m(int dtype, bool friction, bool with_tape, const void* z0, const void* theta, const double* tg, int B, int T,
-                         const KOpts& ko, void* traj, int32_t* ret, int32_t* na, int32_t* nr, const TapeView<float>& tv,
-                         const GridInfo& gi, cudaStream_t s) {
-    return dtype == LDEQ_F32 ? fwd_s<M, float>(friction, with_tape, z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s)
-                             : fwd_s<M, double>(friction, with_tape, z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s);
-}
-
-cudaError_t launch_erk_fwd(int solver, int dtype, bool friction, bool with_tape, const void* z0, const void* theta, const double* tg, int B,
-                           int T, const KOpts& ko, void* traj, int32_t* ret, int32_t* na, int32_t* nr, const TapeView<float>& tv,
-                           const GridInfo& gi, cudaStream_t s) {
-    switch (solver) {
-        case LDEQ_SOLVER_DP5: return fwd_m<DP5M>(dtype, friction, with_tape, z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s);
-        case LDEQ_SOLVER_BS3: return fwd_m<BS3M>(dtype, friction, with_tape, z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s);
-        case LDEQ_SOLVER_RK4: return fwd_m<RK4M>(dtype, friction, with_tape, z0, theta, tg, B, T, ko, traj, ret, na, nr, tv, gi, s);
-        default: return cudaErrorInvalidValue;
-    }
-}
-
 template <class M, class S, bool FRICTION>
-static cudaError_t bwd_t(const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    TapeView<S> tv{tape->t, (S*)tape->u, tape->info, tape->cap, nullptr, nullptr, nullptr, nullptr, nullptr};
-    const int grid = (tape->B + LDEQ_BWD_THREADS - 1) / LDEQ_BWD_THREADS;
-    const size_t smem = Ring<S, 2>::bytes(LDEQ_BWD_THREADS) + (tape->T <= LDEQ_TGRID_SMEM_MAX ? (size_t)tape->T * sizeof(double) : 0);
-    erk_bwd_kernel<M, PendulumRHS<S, FRICTION>, S><<<grid, LDEQ_BWD_THREADS, smem, s>>>(
-        (const S*)tape->theta, tape->tgrid, tape->B, tape->T, (const S*)dtraj, tv, tape->retcode, tape->naccept, (S*)dz0, (S*)dtheta,
-        GridInfo{tape->grid_t0, tape->grid_h, tape->grid_uniform, ld, bwd_sort_lanes()});
-    return cudaGetLastError();
+static void fill(GokuKernels& k, int dtype) {
+    k.fwd[dtype][0] = (void*)erk_fwd_kernel<M, PendulumRHS<S, FRICTION>, S, false>;
+    k.fwd[dtype][1] = (void*)erk_fwd_kernel<M, PendulumRHS<S, FRICTION>, S, true>;
+    k.bwd[dtype] = (void*)erk_bwd_kernel<M, PendulumRHS<S, FRICTION>, S>;
 }
 
-template <class M>
-static cudaError_t bwd_m(const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    const bool fr = tape->rhs_kind == LDEQ_RHS_PENDULUM_FRICTION;
-    if (tape->dtype == LDEQ_F32)
-        return fr ? bwd_t<M, float, true>(tape, dtraj, ld, dz0, dtheta, s) : bwd_t<M, float, false>(tape, dtraj, ld, dz0, dtheta, s);
-    return fr ? bwd_t<M, double, true>(tape, dtraj, ld, dz0, dtheta, s) : bwd_t<M, double, false>(tape, dtraj, ld, dz0, dtheta, s);
+template <bool FRICTION>
+static void fill_solvers(GokuKernels* k) {
+    fill<Tsit5M, float, FRICTION>(k[LDEQ_SOLVER_TSIT5], LDEQ_F32);
+    fill<Tsit5M, double, FRICTION>(k[LDEQ_SOLVER_TSIT5], LDEQ_F64);
+    fill<DP5M, float, FRICTION>(k[LDEQ_SOLVER_DP5], LDEQ_F32);
+    fill<DP5M, double, FRICTION>(k[LDEQ_SOLVER_DP5], LDEQ_F64);
+    fill<BS3M, float, FRICTION>(k[LDEQ_SOLVER_BS3], LDEQ_F32);
+    fill<BS3M, double, FRICTION>(k[LDEQ_SOLVER_BS3], LDEQ_F64);
+    fill<RK4M, float, FRICTION>(k[LDEQ_SOLVER_RK4], LDEQ_F32);
+    fill<RK4M, double, FRICTION>(k[LDEQ_SOLVER_RK4], LDEQ_F64);
 }
 
-cudaError_t launch_erk_bwd(const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    switch (tape->solver) {
-        case LDEQ_SOLVER_DP5: return bwd_m<DP5M>(tape, dtraj, ld, dz0, dtheta, s);
-        case LDEQ_SOLVER_BS3: return bwd_m<BS3M>(tape, dtraj, ld, dz0, dtheta, s);
-        case LDEQ_SOLVER_RK4: return bwd_m<RK4M>(tape, dtraj, ld, dz0, dtheta, s);
-        default: return cudaErrorInvalidValue;
-    }
+void builtin_solve_kernels(int kind, GokuKernels* k) {
+    if (kind == LDEQ_RHS_PENDULUM_FRICTION) fill_solvers<true>(k);
+    else fill_solvers<false>(k);
 }
 
 }  // namespace ldeq

@@ -5,33 +5,10 @@
 
 namespace ldeq {
 
-template <class MD, class S, bool FR>
-static cudaError_t launch_t(const ldeq_tape* tp, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    const int B = tp->B, grid = (B + LDEQ_FWDSENS_THREADS - 1) / LDEQ_FWDSENS_THREADS;
-    const GridInfo gi{tp->grid_t0, tp->grid_h, tp->grid_uniform, ld};
-    const int* key = fwdsens_sort_key(tp);
-    erk_fwdsens_kernel<MD, S, 1, FR, true><<<grid, LDEQ_FWDSENS_THREADS, 0, s>>>((const S*)tp->u, (const S*)tp->theta, tp->tgrid, B, gi, tp->T, tp->kopts,
-                                                                                1, key, (const S*)dtraj, tp->retcode, (S*)dtheta);
-    erk_fwdsens_kernel<MD, S, 2, FR, false><<<grid, LDEQ_FWDSENS_THREADS, 0, s>>>((const S*)tp->u, (const S*)tp->theta, tp->tgrid, B, gi, tp->T, tp->kopts,
-                                                                                 1, key, (const S*)dtraj, tp->retcode, (S*)dz0);
-    return cudaGetLastError();
-}
-
-template <class MD>
-static cudaError_t launch_m(const ldeq_tape* tp, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    const bool fr = tp->rhs_kind == LDEQ_RHS_PENDULUM_FRICTION;
-    if (tp->dtype == LDEQ_F32)
-        return fr ? launch_t<MD, float, true>(tp, dtraj, ld, dz0, dtheta, s) : launch_t<MD, float, false>(tp, dtraj, ld, dz0, dtheta, s);
-    return fr ? launch_t<MD, double, true>(tp, dtraj, ld, dz0, dtheta, s) : launch_t<MD, double, false>(tp, dtraj, ld, dz0, dtheta, s);
-}
-
-cudaError_t launch_erk_fwdsens(const ldeq_tape* tp, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    switch (tp->solver) {
-        case LDEQ_SOLVER_DP5: return launch_m<ErkDual<TabDP5>>(tp, dtraj, ld, dz0, dtheta, s);
-        case LDEQ_SOLVER_BS3: return launch_m<ErkDual<TabBS3>>(tp, dtraj, ld, dz0, dtheta, s);
-        case LDEQ_SOLVER_RK4: return launch_m<ErkDual<TabRK4>>(tp, dtraj, ld, dz0, dtheta, s);
-        default: return cudaErrorInvalidValue;
-    }
+void builtin_fwdsens_erk(int kind, GokuKernels* k) {
+    fill_fwdsens<ErkDual<TabDP5>>(kind, k[LDEQ_SOLVER_DP5]);
+    fill_fwdsens<ErkDual<TabBS3>>(kind, k[LDEQ_SOLVER_BS3]);
+    fill_fwdsens<ErkDual<TabRK4>>(kind, k[LDEQ_SOLVER_RK4]);
 }
 
 }  // namespace ldeq

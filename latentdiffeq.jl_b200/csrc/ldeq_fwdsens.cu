@@ -7,24 +7,6 @@
 
 namespace ldeq {
 
-template <class S, bool FR>
-static cudaError_t launch_fwdsens_t(const ldeq_tape* tp, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    const int B = tp->B, grid = (B + LDEQ_FWDSENS_THREADS - 1) / LDEQ_FWDSENS_THREADS;
-    const GridInfo gi{tp->grid_t0, tp->grid_h, tp->grid_uniform, ld};
-    const int* key = fwdsens_sort_key(tp);
-    tsit5_fwdsens_kernel<S, 1, FR, true><<<grid, LDEQ_FWDSENS_THREADS, 0, s>>>((const S*)tp->u, (const S*)tp->theta, tp->tgrid, B, gi, tp->T, tp->kopts, 1, key,
-                                                             (const S*)dtraj, tp->retcode, (S*)dtheta);
-    tsit5_fwdsens_kernel<S, 2, FR, false><<<grid, LDEQ_FWDSENS_THREADS, 0, s>>>((const S*)tp->u, (const S*)tp->theta, tp->tgrid, B, gi, tp->T, tp->kopts, 1, key,
-                                                              (const S*)dtraj, tp->retcode, (S*)dz0);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_fwdsens(const ldeq_tape* tp, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s) {
-    if (tp->solver != LDEQ_SOLVER_TSIT5) return launch_erk_fwdsens(tp, dtraj, ld, dz0, dtheta, s);
-    const bool fr = tp->rhs_kind == LDEQ_RHS_PENDULUM_FRICTION;
-    if (tp->dtype == LDEQ_F32)
-        return fr ? launch_fwdsens_t<float, true>(tp, dtraj, ld, dz0, dtheta, s) : launch_fwdsens_t<float, false>(tp, dtraj, ld, dz0, dtheta, s);
-    return fr ? launch_fwdsens_t<double, true>(tp, dtraj, ld, dz0, dtheta, s) : launch_fwdsens_t<double, false>(tp, dtraj, ld, dz0, dtheta, s);
-}
+void builtin_fwdsens_tsit5(int kind, GokuKernels* k) { fill_fwdsens<Tsit5Dual>(kind, k[LDEQ_SOLVER_TSIT5]); }
 
 }  // namespace ldeq

@@ -4,7 +4,7 @@
 // Pullback per trajectory: seed theta with Dual partials and re-solve, dtheta = sum_k (du_k/dtheta)^T Delta_k; seed u0
 // and re-solve, dz0 likewise.  The error norm of a Dual state includes the partials (sse(value) + sum sse(partials),
 // partials counted as entries), so each dual solve takes its OWN accepted-step sequence -- this is what makes the
-// reference's gradient differ from the discrete adjoint of the primal steps (tsit5_bwd_kernel) by up to the solver
+// reference's gradient differ from the discrete adjoint of the primal steps (erk_bwd_kernel) by up to the solver
 // tolerance.  The body restates that algorithm literally, including Julia's arithmetic promotion (a Float32 state
 // meets the Float64 dt: `uprev + dt*(...)` is evaluated in Float64 and rounded on the store; the dense-output
 // polynomials are evaluated in Float64), so that its step sequences are the oracle's (oracle/ldeq_oracle.cpp::solve_one
@@ -375,15 +375,6 @@ erk_fwdsens_body(const S* __restrict__ z0, const S* __restrict__ theta, const do
     const bool ok = ret == RET_SUCCESS && primal_ret[b] == RET_SUCCESS;
 #pragma unroll
     for (int q = 0; q < NP; ++q) dout[(size_t)b * NP + q] = ok ? (S)acc[q] : (S)0;
-}
-
-// the Tsit5 instantiation under its own name (NVRTC wrapper source)
-template <class RHS, class S, int NP, bool SEED_P>
-__device__ __forceinline__ void
-tsit5_fwdsens_body(const S* __restrict__ z0, const S* __restrict__ theta, const double* __restrict__ tg, int B, GridInfo gi, int T,
-                   KOpts o, int norm_partials, const int* __restrict__ sort_key, const S* __restrict__ dtraj, const int* __restrict__ primal_ret,
-                   S* __restrict__ dout) {
-    erk_fwdsens_body<Tsit5Dual, RHS, S, NP, SEED_P>(z0, theta, tg, B, gi, T, o, norm_partials, sort_key, dtraj, primal_ret, dout);
 }
 
 }  // namespace ldeq

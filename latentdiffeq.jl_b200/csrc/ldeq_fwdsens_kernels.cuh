@@ -3,7 +3,6 @@
 #pragma once
 #include "ldeq_internal.h"
 #include "ldeq_fwdsens.cuh"
-#include <cstdlib>
 
 #ifndef LDEQ_FWDSENS_MINBLOCKS
 // 5 CTAs of 128 threads per SM (<= 102 registers; the u0-seeded Float32 kernel spills 80 bytes): measured 6.20 -> 5.93 ms for
@@ -38,15 +37,7 @@ template <bool FRICTION> struct PendulumDualRHS {
     }
 };
 
-template <class S, int NP, bool FRICTION, bool SEED_P>
-__global__ void __launch_bounds__(LDEQ_FWDSENS_THREADS, LDEQ_FWDSENS_MINBLOCKS)
-tsit5_fwdsens_kernel(const S* __restrict__ z0, const S* __restrict__ theta, const double* __restrict__ tg, int B, GridInfo gi, int T,
-                     KOpts o, int norm_partials, const int* __restrict__ sort_key, const S* __restrict__ dtraj, const int* __restrict__ primal_ret,
-                     S* __restrict__ dout) {
-    tsit5_fwdsens_body<PendulumDualRHS<FRICTION>, S, NP, SEED_P>(z0, theta, tg, B, gi, T, o, norm_partials, sort_key, dtraj, primal_ret, dout);
-}
-
-// the same for the table-driven methods (MD = ErkDual<TabDP5> ...)
+// MD: the method on duals, Tsit5Dual or ErkDual<TabDP5> ...
 template <class MD, class S, int NP, bool FRICTION, bool SEED_P>
 __global__ void __launch_bounds__(LDEQ_FWDSENS_THREADS, LDEQ_FWDSENS_MINBLOCKS)
 erk_fwdsens_kernel(const S* __restrict__ z0, const S* __restrict__ theta, const double* __restrict__ tg, int B, GridInfo gi, int T,
@@ -55,10 +46,18 @@ erk_fwdsens_kernel(const S* __restrict__ z0, const S* __restrict__ theta, const 
     erk_fwdsens_body<MD, PendulumDualRHS<FRICTION>, S, NP, SEED_P>(z0, theta, tg, B, gi, T, o, norm_partials, sort_key, dtraj, primal_ret, dout);
 }
 
-// LDEQ_FWDSENS_SORT=0 keeps the trajectory -> lane assignment of the batch order (A/B switch; the results are identical)
-inline const int* fwdsens_sort_key(const ldeq_tape* tp) {
-    static const bool sort = [] { const char* e = getenv("LDEQ_FWDSENS_SORT"); return !(e && e[0] == '0'); }();
-    return sort ? tp->naccept : nullptr;
+// the pullback entries of the kernel table of method MD
+template <class MD, bool FRICTION>
+void fill_fwdsens(GokuKernels& k) {
+    k.fwdsens[LDEQ_F32][0] = (void*)erk_fwdsens_kernel<MD, float, 1, FRICTION, true>;
+    k.fwdsens[LDEQ_F32][1] = (void*)erk_fwdsens_kernel<MD, float, 2, FRICTION, false>;
+    k.fwdsens[LDEQ_F64][0] = (void*)erk_fwdsens_kernel<MD, double, 1, FRICTION, true>;
+    k.fwdsens[LDEQ_F64][1] = (void*)erk_fwdsens_kernel<MD, double, 2, FRICTION, false>;
+}
+template <class MD>
+void fill_fwdsens(int kind, GokuKernels& k) {
+    if (kind == LDEQ_RHS_PENDULUM_FRICTION) fill_fwdsens<MD, true>(k);
+    else fill_fwdsens<MD, false>(k);
 }
 
 }  // namespace ldeq

@@ -65,19 +65,28 @@ struct ldeq_handle {
     cudaEvent_t ev_fwd[LDEQ_MAX_SLABS] = {}, ev_up[LDEQ_MAX_SLABS] = {}, ev_join = nullptr;
 };
 
+namespace ldeq {
+// The kernels of one right-hand side under one solver, indexed by ldeq_dtype.  Every GOKU solve is one launch of an entry
+// (two for the pullback), whatever the right-hand side: the built-ins fill their tables in ldeq_rhs_builtin, a user RHS
+// from its NVRTC module (ldeq_user_rhs.cu).
+struct GokuKernels {
+    void* fwd[2][2] = {};      // forward solve [f32, f64][no tape, tape]
+    void* bwd[2] = {};         // discrete adjoint [f32, f64]
+    void* fwdsens[2][2] = {};  // forward-dual pullback [f32, f64][theta-seeded, u0-seeded]
+};
+}  // namespace ldeq
+
 struct ldeq_rhs {
-    int kind = 0;  // ldeq_rhs_kind, or -1 for an NVRTC-compiled user RHS
     int z_dim = 2, p_dim = 1;
-    void* module = nullptr;  // CUmodule of a user RHS
-    void* fn[12] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    // a user RHS under another `solver`: its own NVRTC module, compiled on first use from the kept source
-    struct PerSolver { void* module = nullptr; void* fn[12] = {}; };
-    PerSolver alt[4];
+    // one table per ldeq_solver; a user RHS compiles the table of a solver on first use (ldeq::rhs_kernels)
+    ldeq::GokuKernels kernels[4];
+    void* module[4] = {};  // cudaLibrary_t of each compiled variant of a user RHS
     std::string user_src;
+    bool built(int solver) const { return kernels[solver].fwd[0][0] != nullptr; }
 };
 
 struct ldeq_tape {
-    int dtype = 0, rhs_kind = 0, B = 0, T = 0, z_dim = 2, p_dim = 1, cap = 0;
+    int dtype = 0, B = 0, T = 0, z_dim = 2, p_dim = 1, cap = 0;
     const ldeq_rhs* rhs = nullptr;
     void* base = nullptr;  // one stream-ordered allocation, carved into the arrays below
     double* t = nullptr;
@@ -114,17 +123,17 @@ int upload_tgrid(ldeq_handle* h, const double* t_host, int T, cudaStream_t s);
 // grows scratch[slot] to `bytes` on `s`; under capture it refuses to grow (LDEQ_ERR_UNSUPPORTED) and marks the slot captured
 int ensure_scratch(ldeq_handle* h, int slot, size_t bytes, cudaStream_t s);
 KOpts to_kopts(const ldeq_opts* o);
-int bwd_sort_lanes();  // ldeq_api.cu: lane re-deal of the discrete-adjoint kernels (LDEQ_BWD_SORT)
 // pooled pinned {int32 x 2} mirror + event (ldeq_api.cu)
 bool slot_acquire(ldeq_handle* h, int32_t** h_info, cudaEvent_t* ev);
 void slot_release(ldeq_handle* h, int32_t* h_info, cudaEvent_t ev);
-// ldeq_fwdsens.cu: the reference's ForwardDiffSensitivity pullback (two dual-number re-solves per trajectory)
-cudaError_t launch_fwdsens(const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s);
-// ldeq_erk_fwdsens.cu / ldeq_erk.cu: the same kernels for solver = DP5 / BS3 / RK4 (built-in right-hand sides)
-cudaError_t launch_erk_fwdsens(const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s);
-cudaError_t launch_erk_bwd(const ldeq_tape* tape, const void* dtraj, int ld, void* dz0, void* dtheta, cudaStream_t s);
-// ldeq_user_rhs.cu: kernel table of a user RHS for `solver` (compiles the variant on first use); null + error text on failure
-void* const* user_rhs_kernels(ldeq_handle* h, const ldeq_rhs* rhs, int solver);
+// The kernel tables of the built-in right-hand side `kind`, k[ldeq_solver], filled pass by pass by the translation unit
+// that compiles it: ldeq_erk.cu the forward solve and the discrete adjoint, ldeq_fwdsens.cu (Tsit5) and
+// ldeq_erk_fwdsens.cu (DP5, BS3, RK4) the forward-dual pullback.
+void builtin_solve_kernels(int kind, GokuKernels* k);
+void builtin_fwdsens_tsit5(int kind, GokuKernels* k);
+void builtin_fwdsens_erk(int kind, GokuKernels* k);
+// ldeq_user_rhs.cu: the kernel table of `rhs` for `solver` (a user RHS compiles it on first use); null + error text on failure
+const GokuKernels* rhs_kernels(ldeq_handle* h, const ldeq_rhs* rhs, int solver);
 
 #define LDEQ_CUDA(call)                                                    \
     do {                                                                   \

@@ -380,7 +380,7 @@ mlp_tc_adj_kernel(TcNet net, const unsigned char* __restrict__ img_global, const
                 tc_ld8(R0 + c0, gb);
 #pragma unroll
                 for (int i = 0; i < 8; ++i) gb[i] = (valid && c0 + i < D) ? gb[i] : 0.f;
-                // Tsit5 adjoint bookkeeping (stage st+1; mirrors tsit5_bwd_body of ldeq_tsit5.cuh)
+                // Tsit5 adjoint bookkeeping (stage st+1; mirrors erk_bwd_body of ldeq_tsit5.cuh)
                 if (st == 6) {
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {

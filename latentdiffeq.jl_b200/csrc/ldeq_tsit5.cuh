@@ -777,39 +777,7 @@ erk_bwd_body(const S* __restrict__ theta, const double* __restrict__ tg_global, 
 }
 
 // ---- kernel entry points ---------------------------------------------------------------------------------
-// the Tsit5 instantiations under their own names (NVRTC wrapper source, launch lists in profiles/)
-template <class RHS, class S, bool TAPE>
-__device__ __forceinline__ void
-tsit5_fwd_body(const S* __restrict__ z0, const S* __restrict__ theta, const double* __restrict__ tg_global, int B,
-               int T, KOpts o, S* __restrict__ traj, int* __restrict__ retcode, int* __restrict__ naccept,
-               int* __restrict__ nreject, TapeView<S> tape, GridInfo ginfo) {
-    erk_fwd_body<Tsit5M, RHS, S, TAPE>(z0, theta, tg_global, B, T, o, traj, retcode, naccept, nreject, tape, ginfo);
-}
-template <class RHS, class S>
-__device__ __forceinline__ void
-tsit5_bwd_body(const S* __restrict__ theta, const double* __restrict__ tg_global, int B, int T,
-               const S* __restrict__ dtraj, TapeView<S> tape, const int* __restrict__ retcode,
-               const int* __restrict__ naccept, S* __restrict__ dz0, S* __restrict__ dtheta, GridInfo ginfo) {
-    erk_bwd_body<Tsit5M, RHS, S>(theta, tg_global, B, T, dtraj, tape, retcode, naccept, dz0, dtheta, ginfo);
-}
-
-template <class RHS, class S, bool TAPE>
-__global__ void __launch_bounds__(LDEQ_FWD_THREADS, LDEQ_FWD_MINBLOCKS)
-tsit5_fwd_kernel(const S* __restrict__ z0, const S* __restrict__ theta, const double* __restrict__ tg_global, int B,
-                 int T, KOpts o, S* __restrict__ traj, int* __restrict__ retcode, int* __restrict__ naccept,
-                 int* __restrict__ nreject, TapeView<S> tape, GridInfo ginfo) {
-    tsit5_fwd_body<RHS, S, TAPE>(z0, theta, tg_global, B, T, o, traj, retcode, naccept, nreject, tape, ginfo);
-}
-
-template <class RHS, class S>
-__global__ void __launch_bounds__(LDEQ_BWD_THREADS, LDEQ_BWD_MINBLOCKS)
-tsit5_bwd_kernel(const S* __restrict__ theta, const double* __restrict__ tg_global, int B, int T,
-                 const S* __restrict__ dtraj, TapeView<S> tape, const int* __restrict__ retcode,
-                 const int* __restrict__ naccept, S* __restrict__ dz0, S* __restrict__ dtheta, GridInfo ginfo) {
-    tsit5_bwd_body<RHS, S>(theta, tg_global, B, T, dtraj, tape, retcode, naccept, dz0, dtheta, ginfo);
-}
-
-// the same kernels for the table-driven methods (M = DP5M / BS3M / RK4M, ldeq_erk.cuh)
+// M: the method, Tsit5M or the table-driven DP5M / BS3M / RK4M (ldeq_erk.cuh)
 template <class M, class RHS, class S, bool TAPE>
 __global__ void __launch_bounds__(LDEQ_FWD_THREADS, LDEQ_FWD_MINBLOCKS)
 erk_fwd_kernel(const S* __restrict__ z0, const S* __restrict__ theta, const double* __restrict__ tg_global, int B,
