@@ -36,7 +36,8 @@
  *   graph, so per-step values go through the _dev entry points below, which read them from device memory.
  *   Capture-safe: ldeq_solve_fwd (no tape, or a FORWARD_DUAL tape) and ldeq_solve_bwd of such a tape, ldeq_tape_free,
  *   ldeq_pattern_extractor_fwd / _bwd / ldeq_pe_tape_free, ldeq_sample / _dev, ldeq_elbo_* / _dev, ldeq_adamw_step /
- *   _dev.  Rules:
+ *   _dev, ldeq_mlp_solve_fwd_dev (no tape, or a device-checked tape other than INTERPOLATING_ADJOINT), ldeq_mlp_solve_bwd of
+ *   such a tape and ldeq_mlp_tape_free.  Rules:
  *   - A tape recorded under capture has no host mirror and no event: its allocation and release become graph nodes.
  *   - A captured solve reads an immutable device copy of its time grid, kept by the handle until ldeq_destroy (the grid
  *     an eager call uses is overwritten when another grid arrives).  The copy is made by an eager solve on the same grid:
@@ -45,8 +46,8 @@
  *     non-Tsit5 solver are created by a first eager call; under capture their absence is refused.
  *   - Refused with LDEQ_ERR_UNSUPPORTED, before anything is enqueued (the capture stays valid and can be ended), because
  *     they need the host while the work runs: a DISCRETE_ADJOINT tape and its reverse pass (the tape's overflow check,
- *     tape_heal), ldeq_tape_overflow, ldeq_mlp_solve_fwd / _bwd and ldeq_mlp_bwd_stats (the MLP tape check and the
- *     continuous adjoint), every _host entry point (staging and stream synchronisation), ldeq_allreduce_grads and
+ *     tape_heal), ldeq_tape_overflow, ldeq_mlp_solve_fwd, ldeq_mlp_solve_bwd of its tape and ldeq_mlp_bwd_stats (the MLP
+ *     tape check on the host and the continuous adjoint), every _host entry point (staging and stream synchronisation), ldeq_allreduce_grads and
  *     ldeq_allreduce_adamw_step (multi-GPU capture is not built).  ldeq_comm_unique_id / _init / _destroy take no stream:
  *     they are set-up calls that synchronise the device and must not be made while a capture is open.
  */
@@ -235,6 +236,25 @@ int ldeq_mlp_solve_fwd(ldeq_handle* h, int dtype, const void* z0, const void* pa
                        const int32_t* layer_dims_host, int n_layers, const double* t_host, int B, int T,
                        const ldeq_opts* opts, void* traj_out, int32_t* retcode, int32_t* naccept,
                        int32_t* nreject, ldeq_mlp_tape** tape_out, ldeq_stream stream);
+/* The same solve with a DEVICE-CHECKED tape, for CUDA graphs (a training step of LatentODE.jl:61-78 captured once and
+ * replayed): same checks, same kernels, the same traj / retcode / naccept / nreject and tape contents bit for bit, eagerly
+ * and under capture.  The tape takes no pinned host mirror or event and its pullback never waits for the host: where the
+ * tape of ldeq_mlp_solve_fwd makes ldeq_mlp_solve_bwd return LDEQ_ERR_TAPE_OVERFLOW (more accepted steps N than
+ * opts->tape_steps), this one's pullback writes NaN into the overflowed rows of dz0 (as both do) and into EVERY element of
+ * dparams_flat, and raises the caller-owned device word *overflow to max(*overflow, N) -- the tape_steps to ask for.  The
+ * word is sticky: only the caller clears it.  The pullback of a tape whose steps all fit writes exactly what the pullback
+ * of the ldeq_mlp_solve_fwd tape writes.  A tape needs a non-null `overflow` (LDEQ_ERR_INVALID otherwise).
+ * Refused with LDEQ_ERR_UNSUPPORTED before anything is enqueued: a tape for LDEQ_SENSE_INTERPOLATING_ADJOINT (the continuous
+ * adjoint sizes its dense output from the host count), and under capture a grid no eager solve has brought to the device or
+ * device scratch that would have to grow.  A BF16X3 tape's reverse pass keeps tape_steps step records per 128 trajectories
+ * (about 3 MB each for the reference's 16-200-200-16 network): this call allocates them, or refuses with their size. */
+int ldeq_mlp_solve_fwd_dev(ldeq_handle* h, int dtype, const void* z0, const void* params_flat,
+                           const int32_t* layer_dims_host, int n_layers, const double* t_host, int B, int T,
+                           const ldeq_opts* opts, void* traj_out, int32_t* retcode, int32_t* naccept,
+                           int32_t* nreject, int32_t* overflow /* device word, caller-owned */,
+                           ldeq_mlp_tape** tape_out, ldeq_stream stream);
+/* The pullback of either tape.  An ldeq_mlp_solve_fwd tape: waits for its forward kernel, returns LDEQ_ERR_TAPE_OVERFLOW
+ * when the tape was too short, and is refused under capture.  A device-checked tape: capture-safe, never waits. */
 int ldeq_mlp_solve_bwd(ldeq_handle* h, ldeq_mlp_tape* tape, const void* dtraj, void* dz0,
                        void* dparams_flat, ldeq_stream stream);
 /* {accepted steps, rejected steps, retcode} of the backward solve that LDEQ_SENSE_INTERPOLATING_ADJOINT ran for this

@@ -13,7 +13,7 @@ from ._cabi import (F32, F64, RHS_PENDULUM, RHS_PENDULUM_FRICTION, RET_SUCCESS, 
                     RET_UNSTABLE, NORM_GLOBAL, NORM_PER_TRAJ, MLP_MATH_FP32, MLP_MATH_BF16X3, LdeqError, default_opts,
                     handle, Handle, SOLVER_TSIT5, SOLVER_DP5, SOLVER_BS3, SOLVER_RK4, SENSE_DISCRETE_ADJOINT, SENSE_FORWARD_DUAL, SENSE_INTERPOLATING_ADJOINT)
 from .solve import (goku_solve, goku_solve_raw, goku_bwd_raw, goku_solve_host, goku_bwd_host, goku_fwd_bwd_host, debug_trig, mlp_solve, mlp_solve_raw,
-                    mlp_bwd_raw, mlp_bwd_stats, pattern_extractor, pe_flat_params, sample_raw, sample_reparam, elbo_raw, elbo_loss, adamw_step, adamw_step_dev, adamw_state,
+                    mlp_bwd_raw, device_tape_check, mlp_bwd_stats, pattern_extractor, pe_flat_params, sample_raw, sample_reparam, elbo_raw, elbo_loss, adamw_step, adamw_step_dev, adamw_state,
                     allreduce_adamw_step)
 from .diffeqs import (Tsit5, DP5, BS3, RK4, ForwardDiffSensitivity, DiscreteAdjoint, InterpolatingAdjoint, ODEProblem, CudaRHS, Pendulum, Pendulum_friction,
                       UserDiffEq, NODE)

@@ -29,7 +29,7 @@ SYMBOLS = [
     "ldeq_mlp_solve_fwd", "ldeq_mlp_solve_bwd", "ldeq_mlp_tape_free", "ldeq_mlp_bwd_stats", "ldeq_debug_cadj_trace",
     "ldeq_pattern_extractor_param_count", "ldeq_pattern_extractor_fwd", "ldeq_pattern_extractor_bwd", "ldeq_pe_tape_free",
     "ldeq_sample", "ldeq_elbo_fwd_bwd", "ldeq_elbo_logits_fwd_bwd", "ldeq_adamw_step", "ldeq_allreduce_adamw_step",
-    "ldeq_sample_dev", "ldeq_elbo_fwd_bwd_dev", "ldeq_elbo_logits_fwd_bwd_dev", "ldeq_adamw_step_dev",
+    "ldeq_sample_dev", "ldeq_elbo_fwd_bwd_dev", "ldeq_elbo_logits_fwd_bwd_dev", "ldeq_adamw_step_dev", "ldeq_mlp_solve_fwd_dev",
     "ldeq_comm_unique_id", "ldeq_comm_init", "ldeq_allreduce_grads", "ldeq_comm_destroy",
 ]
 COMM_ID_BYTES = 128
@@ -96,6 +96,7 @@ def load() -> C.CDLL:
     lib.ldeq_solve_fwd_bwd_host.argtypes = [vp, vp, i32, vp, vp, vp, i32, i32, C.POINTER(Opts), vp, vp, vp, vp, vp, vp, vp, vp]
     lib.ldeq_debug_trig.argtypes = [vp, i32, vp, vp, vp, i64, vp]
     lib.ldeq_mlp_solve_fwd.argtypes = [vp, i32, vp, vp, vp, i32, vp, i32, i32, C.POINTER(Opts), vp, vp, vp, vp, pvp, vp]
+    lib.ldeq_mlp_solve_fwd_dev.argtypes = [vp, i32, vp, vp, vp, i32, vp, i32, i32, C.POINTER(Opts), vp, vp, vp, vp, vp, pvp, vp]
     lib.ldeq_mlp_solve_bwd.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.ldeq_mlp_bwd_stats.argtypes = [vp, vp, vp, vp]
     lib.ldeq_debug_cadj_trace.argtypes = [vp, vp, vp, C.c_int]

@@ -95,6 +95,34 @@ int upload_tgrid(ldeq_handle* h, const double* t_host, int T, cudaStream_t s) {
     return LDEQ_OK;
 }
 
+int captured_grid(ldeq_handle* h, const double* t_host, int T, const char* who, GridRef* out) {
+    ldeq_handle::GridEntry* g = nullptr;
+    for (auto& e : h->grid_cache)
+        if (same_grid(e.t, t_host, T)) { g = &e; break; }
+    if (!g) {
+        std::string msg = std::string(who) + ": the time grid is not on the device, and a copy from host memory cannot be captured: "
+                                             "solve once on this grid outside the capture first";
+        return set_err(h, LDEQ_ERR_UNSUPPORTED, msg.c_str());
+    }
+    g->pinned = true;  // the graph reads g->d for as long as the handle lives
+    *out = GridRef{g->d, g->t0, g->h, g->uniform};
+    return LDEQ_OK;
+}
+
+cudaError_t launch_cooperative(const void* fn, dim3 grid, dim3 block, void** args, size_t smem, cudaStream_t s) {
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeCooperative;
+    attr[0].val.cooperative = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelExC(&cfg, fn, args);
+}
+
 int ensure_scratch(ldeq_handle* h, int slot, size_t bytes, cudaStream_t s) {
     const bool graph = capturing(s);
     if (bytes <= h->scratch_cap[slot]) {
@@ -399,12 +427,6 @@ int ldeq_rhs_dims(const ldeq_rhs* rhs, int* z_dim, int* p_dim) {
 
 namespace ldeq {
 
-// The device grid a solve reads: d_tgrid for eager calls, an immutable cache entry under capture.
-struct GridRef {
-    const double* d;
-    double t0, h;
-    int uniform;
-};
 static GridRef eager_grid(const ldeq_handle* h) { return GridRef{h->d_tgrid, h->grid_t0, h->grid_h, h->grid_uniform}; }
 
 // ---- one column slab of a solve -----------------------------------------------------------------------
@@ -597,15 +619,9 @@ int ldeq_solve_fwd(ldeq_handle* h, const ldeq_rhs* rhs, int dtype, const void* z
     if (!rhs->built(opts->solver))
         return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_fwd: the right-hand side has not been compiled for this solver yet, and NVRTC "
                                                 "cannot run under CUDA graph capture: solve once outside the capture first");
-    ldeq_handle::GridEntry* g = nullptr;
-    for (auto& e : h->grid_cache)
-        if (same_grid(e.t, t_host, T)) { g = &e; break; }
-    if (!g)
-        return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_solve_fwd: the time grid is not on the device, and a copy from host memory cannot be "
-                                                "captured: solve once on this grid outside the capture first");
-    g->pinned = true;  // the graph reads g->d for as long as the handle lives
-    return solve_fwd_slab(h, rhs, dtype, z0, theta, t_host, GridRef{g->d, g->t0, g->h, g->uniform}, true, B, B, T, opts, traj_out, retcode,
-                          naccept, nreject, tape_out, s);
+    GridRef grid;
+    if ((rc = captured_grid(h, t_host, T, "ldeq_solve_fwd", &grid))) return rc;
+    return solve_fwd_slab(h, rhs, dtype, z0, theta, t_host, grid, true, B, B, T, opts, traj_out, retcode, naccept, nreject, tape_out, s);
 }
 
 int ldeq_solve_bwd(ldeq_handle* h, ldeq_tape* tape, const void* dtraj, void* dz0, void* dtheta, ldeq_stream stream) {

@@ -120,6 +120,18 @@ bool capturing(cudaStream_t s);
 // LDEQ_ERR_UNSUPPORTED with "<what>: not available under CUDA graph capture (<why>)" when `s` is capturing, else LDEQ_OK.
 int refuse_capture(ldeq_handle* h, cudaStream_t s, const char* what, const char* why);
 int upload_tgrid(ldeq_handle* h, const double* t_host, int T, cudaStream_t s);
+// The device grid a solve reads: d_tgrid for eager calls, an immutable cache entry under capture.
+struct GridRef {
+    const double* d;
+    double t0, h;
+    int uniform;
+};
+// For a solve under capture: the grid_cache entry of t_host, pinned (the graph reads it for as long as the handle lives).
+// Enqueues nothing.  A grid no eager solve has brought to the device is refused (LDEQ_ERR_UNSUPPORTED, naming `who`).
+int captured_grid(ldeq_handle* h, const double* t_host, int T, const char* who, GridRef* out);
+// A cooperative launch (all CTAs co-resident, grid-wide barriers) through cudaLaunchKernelEx with
+// cudaLaunchAttributeCooperative: the same launch eagerly and as a node of a captured CUDA graph.
+cudaError_t launch_cooperative(const void* fn, dim3 grid, dim3 block, void** args, size_t smem, cudaStream_t s);
 // grows scratch[slot] to `bytes` on `s`; under capture it refuses to grow (LDEQ_ERR_UNSUPPORTED) and marks the slot captured
 int ensure_scratch(ldeq_handle* h, int slot, size_t bytes, cudaStream_t s);
 KOpts to_kopts(const ldeq_opts* o);
@@ -134,6 +146,17 @@ void builtin_fwdsens_tsit5(int kind, GokuKernels* k);
 void builtin_fwdsens_erk(int kind, GokuKernels* k);
 // ldeq_user_rhs.cu: the kernel table of `rhs` for `solver` (a user RHS compiles it on first use); null + error text on failure
 const GokuKernels* rhs_kernels(ldeq_handle* h, const ldeq_rhs* rhs, int solver);
+
+// The overflow rule of a device-checked MLP tape (ldeq_mlp_solve_fwd_dev), applied by the kernels that reduce its parameter
+// gradient.  overflow == null (an eager tape): false, nothing is read.  Otherwise: whether the largest accepted-step count
+// info[0] exceeds the tape's capacity -- one device word, so the answer is the same for every thread of the grid -- and
+// thread 0 of block 0 raises *overflow to info[0] (sticky: only the caller clears it).
+__device__ __forceinline__ bool mlp_tape_overflowed(const int32_t* info, int cap, int32_t* overflow) {
+    if (!overflow) return false;
+    const int32_t n = *info;
+    if (n > cap && blockIdx.x == 0 && threadIdx.x == 0) atomicMax(overflow, n);
+    return n > cap;
+}
 
 #define LDEQ_CUDA(call)                                                    \
     do {                                                                   \

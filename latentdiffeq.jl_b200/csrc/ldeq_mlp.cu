@@ -305,10 +305,13 @@ template <class S> __global__ void mlp_transpose_kernel(MlpNet net, const S* __r
     }
 }
 
-// dparams[i] = sum over CTAs of their private accumulators, in a fixed order (deterministic)
+// dparams[i] = sum over CTAs of their private accumulators, in a fixed order (deterministic); NaN everywhere when a
+// device-checked tape overflowed (mlp_tape_overflowed)
 template <class S> __global__ void mlp_reduce_grads_kernel(const S* __restrict__ gscratch, int n_cta, int n_params,
-                                                            S* __restrict__ dparams) {
+                                                            S* __restrict__ dparams, const int32_t* info, int cap, int32_t* overflow) {
+    const bool over = mlp_tape_overflowed(info, cap, overflow);
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_params; i += gridDim.x * blockDim.x) {
+        if (over) { dparams[i] = s_nan<S>(); continue; }
         double a = 0.0;
         for (int c = 0; c < n_cta; ++c) a += (double)gscratch[(size_t)c * n_params + i];
         dparams[i] = (S)a;
@@ -333,7 +336,8 @@ using namespace ldeq;
 // ldeq_mlp_tc.cu: the tcgen05 / TMEM forward kernel (LDEQ_MLP_MATH_BF16X3)
 int ldeq_mlp_tc_backward(ldeq_handle* h, const int32_t* dims, int n_layers, const float* params, const double* d_tgrid, int B, int T,
                          const float* dtraj, double* tape_t, double* tape_dt, float* tape_u, int tape_cap, const int32_t* ret,
-                         const int32_t* na, int max_na, float* dz0, float* dparams, cudaStream_t s);
+                         const int32_t* na, int nsteps, const int32_t* info, int32_t* overflow, float* dz0, float* dparams, cudaStream_t s);
+int ldeq_mlp_tc_record_scratch(ldeq_handle* h, const int32_t* dims, int n_layers, int B, int nsteps, size_t* bytes);
 int ldeq_mlp_tc_forward(ldeq_handle* h, const int32_t* dims, int n_layers, const float* params, const float* z0,
                         const double* d_tgrid, int B, int T, const KOpts& ko, int norm_mode, float* traj, int32_t* ret,
                         int32_t* na, int32_t* nr, double* tape_t, double* tape_dt, float* tape_u, int tape_cap,
@@ -356,8 +360,11 @@ struct ldeq_mlp_tape {
     int32_t* naccept = nullptr;
     int32_t* nreject = nullptr;
     int32_t* info = nullptr;     // device: largest accepted-step count of a successful trajectory
-    int32_t* h_info = nullptr;   // pinned host mirror, valid once `ready` has completed
+    int32_t* h_info = nullptr;   // pinned host mirror, valid once `ready` has completed (eager tapes)
     cudaEvent_t ready = nullptr;
+    // device-checked tape (ldeq_mlp_solve_fwd_dev): the caller's overflow word, which the reverse pass raises to info[0] when
+    // the tape was too short; no host mirror and no event.  Null for an eager tape, whose reverse pass checks on the host.
+    int32_t* overflow = nullptr;
 };
 
 // largest naccept among the trajectories that succeeded: what the reverse pass will want to find on the tape
@@ -417,7 +424,7 @@ static int launch_mlp_fwd(ldeq_handle* h, const MlpNet& net, const void* P, cons
     KOpts kov = ko;
     void* args[] = {&netv, &Pp, &zp, &tg, &B, &T, &kov, &tp, &ret, &na, &nr, &tv, &partials};
     if (GLOBAL) {
-        LDEQ_CUDA(cudaLaunchCooperativeKernel((void*)kern, dim3(grid), dim3(MLP_THREADS), args, smem, s));
+        LDEQ_CUDA(launch_cooperative((const void*)kern, dim3(grid), dim3(MLP_THREADS), args, smem, s));
     } else {
         LDEQ_CUDA(cudaLaunchKernel((void*)kern, dim3(grid), dim3(MLP_THREADS), args, smem, s));
     }
@@ -471,16 +478,16 @@ static int mlp_fwd_dispatch(ldeq_handle* h, const MlpNet& net, const void* P, co
     return launch_mlp_fwd<S, 8, false>(h, net, P, z0, tg, B, T, ko, traj, ret, na, nr, tv, partials, grid, s);
 }
 
-extern "C" {
-
-int ldeq_mlp_solve_fwd(ldeq_handle* h, int dtype, const void* z0, const void* params_flat, const int32_t* layer_dims_host,
-                       int n_layers, const double* t_host, int B, int T, const ldeq_opts* opts, void* traj_out,
-                       int32_t* retcode, int32_t* naccept, int32_t* nreject, ldeq_mlp_tape** tape_out,
-                       ldeq_stream stream) {
-    if (!h) return LDEQ_ERR_INVALID;
-    if (tape_out) *tape_out = nullptr;
-    if (int rc0 = refuse_capture(h, (cudaStream_t)stream, "ldeq_mlp_solve_fwd", "its tape records the accepted-step count for a host-side check")) return rc0;
+// Both forward entry points.  overflow == null: ldeq_mlp_solve_fwd, eager only; its tape gets a pinned host mirror of
+// info[0] for the reverse pass's host check.  DEV (ldeq_mlp_solve_fwd_dev): a device-checked tape that remembers `overflow`,
+// no host mirror, no event; under capture the grid is the pinned grid_cache entry and every check is made before anything
+// is enqueued.
+static int mlp_solve_fwd(bool dev, ldeq_handle* h, int dtype, const void* z0, const void* params_flat, const int32_t* layer_dims_host,
+                         int n_layers, const double* t_host, int B, int T, const ldeq_opts* opts, void* traj_out, int32_t* retcode,
+                         int32_t* naccept, int32_t* nreject, int32_t* overflow, ldeq_mlp_tape** tape_out, cudaStream_t s) {
+    const char* who = dev ? "ldeq_mlp_solve_fwd_dev" : "ldeq_mlp_solve_fwd";
     if (!z0 || !params_flat || !layer_dims_host || !t_host || !opts || !traj_out) return set_err(h, LDEQ_ERR_INVALID, "null argument");
+    if (dev && tape_out && !overflow) return set_err(h, LDEQ_ERR_INVALID, "ldeq_mlp_solve_fwd_dev: a tape needs the overflow word");
     if (B < 1 || T < 1) return set_err(h, LDEQ_ERR_INVALID, "B and T must be >= 1");
     if (dtype != LDEQ_F32 && dtype != LDEQ_F64) return set_err(h, LDEQ_ERR_INVALID, "dtype");
     if (!opts->adaptive && !(opts->dt > 0.0)) return set_err(h, LDEQ_ERR_INVALID, "adaptive = 0 needs dt > 0");
@@ -491,12 +498,48 @@ int ldeq_mlp_solve_fwd(ldeq_handle* h, int dtype, const void* z0, const void* pa
     if (opts->mlp_math != LDEQ_MLP_MATH_FP32 && opts->mlp_math != LDEQ_MLP_MATH_BF16X3) return set_err(h, LDEQ_ERR_INVALID, "mlp_math");
     if (opts->mlp_math == LDEQ_MLP_MATH_BF16X3 && dtype != LDEQ_F32)
         return set_err(h, LDEQ_ERR_UNSUPPORTED, "mlp_math BF16X3 (tensor cores) needs a Float32 state; Float64 runs on the exact path");
+    if (dev && tape_out && opts->sensealg == LDEQ_SENSE_INTERPOLATING_ADJOINT)
+        return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_mlp_solve_fwd_dev: an interpolating-adjoint tape is not available for CUDA graph capture "
+                                                "(the continuous adjoint sizes its dense output from the accepted-step count on the host); "
+                                                "use LDEQ_SENSE_DISCRETE_ADJOINT");
     MlpNet net;
     int rc = make_net(h, layer_dims_host, n_layers, &net);
     if (rc) return rc;
-    cudaStream_t s = (cudaStream_t)stream;
     LDEQ_CUDA(cudaSetDevice(h->device));
-    if ((rc = upload_tgrid(h, t_host, T, s))) return rc;
+    const bool graph = dev && capturing(s);
+    long long cap = 0;
+    if (tape_out) {
+        cap = opts->tape_steps;
+        if (cap <= 0) cap = opts->adaptive ? (4LL * T > 256 ? 4LL * T : 256) : (long long)((t_host[T - 1] - t_host[0]) / opts->dt) + 3;
+        if (cap > opts->maxiters) cap = opts->maxiters;
+    }
+    GridRef grid;
+    if (graph) {
+        if ((rc = captured_grid(h, t_host, T, who, &grid))) return rc;
+        if (h->scratch_cap[0] < sizeof(double) * 4096)
+            return set_err(h, LDEQ_ERR_UNSUPPORTED, "ldeq_mlp_solve_fwd_dev: device scratch must grow, which cannot happen under CUDA graph "
+                                                    "capture: run the same call once outside the capture first");
+    }
+    // A device-checked tensor-core tape: its reverse pass keeps cap step records per tile of 128 trajectories (the host
+    // count of an eager tape is not known).  The buffer is made here, so that neither the reverse pass nor a replay of it
+    // can fail for want of it.
+    if (dev && tape_out && opts->mlp_math == LDEQ_MLP_MATH_BF16X3 && !getenv("LDEQ_MLP_TC_BWD_OFF")) {
+        size_t need = 0;
+        if ((rc = ldeq_mlp_tc_record_scratch(h, layer_dims_host, n_layers, B, (int)cap, &need))) return rc;
+        if (need > h->scratch_cap[1]) {
+            char msg[320];
+            snprintf(msg, sizeof msg, "ldeq_mlp_solve_fwd_dev: the tensor-core reverse pass of this tape needs %.3f GB of step records "
+                     "(%d trajectories, tape_steps %lld), %s; lower opts.tape_steps", need * 1e-9, B, cap,
+                     graph ? "which must exist before a CUDA graph capture: run the same call once outside the capture first"
+                           : "which could not be allocated");
+            if (graph) return set_err(h, LDEQ_ERR_UNSUPPORTED, msg);
+            if (ensure_scratch(h, 1, need, s)) return set_err(h, LDEQ_ERR_NOMEM, msg);
+        }
+    }
+    if (!graph) {
+        if ((rc = upload_tgrid(h, t_host, T, s))) return rc;
+        grid = GridRef{h->d_tgrid, h->grid_t0, h->grid_h, h->grid_uniform};
+    }
     KOpts ko = to_kopts(opts);
     const size_t es = dtype == LDEQ_F32 ? 4 : 8;
     const int D = net.dims[0];
@@ -505,10 +548,8 @@ int ldeq_mlp_solve_fwd(ldeq_handle* h, int dtype, const void* z0, const void* pa
         tape = new ldeq_mlp_tape();
         tape->dtype = dtype; tape->B = B; tape->T = T; tape->net = net; tape->math = opts->mlp_math;
         tape->sense = opts->sensealg; tape->norm_mode = opts->norm_mode; tape->kopts = ko;
-        long long cap = opts->tape_steps;
-        if (cap <= 0) cap = opts->adaptive ? (4LL * T > 256 ? 4LL * T : 256) : (long long)((t_host[T - 1] - t_host[0]) / opts->dt) + 3;
-        if (cap > opts->maxiters) cap = opts->maxiters;
         tape->cap = (int)cap;
+        tape->overflow = dev ? overflow : nullptr;
         const size_t nB = B, c = (size_t)cap;
         size_t off = 0;
         const size_t o_t = off; off += al256(c * nB * 8);
@@ -529,41 +570,71 @@ int ldeq_mlp_solve_fwd(ldeq_handle* h, int dtype, const void* z0, const void* pa
         tape->naccept = (int32_t*)(bp + o_na); tape->nreject = (int32_t*)(bp + o_nr);
         tape->info = (int32_t*)(bp + o_info);
         cudaMemsetAsync(tape->info, 0, 32, s);
-        if (!slot_acquire(h, &tape->h_info, &tape->ready)) {
+        if (!dev && !slot_acquire(h, &tape->h_info, &tape->ready)) {
             cudaFreeAsync(tape->base, s);
             delete tape;
             return set_err(h, LDEQ_ERR_NOMEM, "mlp tape host mirror");
         }
         cudaMemcpyAsync(tape->params, params_flat, (size_t)net.n_params * es, cudaMemcpyDeviceToDevice, s);
-        cudaMemcpyAsync(tape->tgrid, h->d_tgrid, (size_t)T * 8, cudaMemcpyDeviceToDevice, s);
+        cudaMemcpyAsync(tape->tgrid, grid.d, (size_t)T * 8, cudaMemcpyDeviceToDevice, s);
     }
     int32_t* d_ret = tape ? tape->retcode : retcode;
     int32_t* d_na = tape ? tape->naccept : naccept;
     int32_t* d_nr = tape ? tape->nreject : nreject;
     if (opts->mlp_math == LDEQ_MLP_MATH_BF16X3)
-        rc = ldeq_mlp_tc_forward(h, layer_dims_host, n_layers, (const float*)params_flat, (const float*)z0, h->d_tgrid, B, T, ko,
+        rc = ldeq_mlp_tc_forward(h, layer_dims_host, n_layers, (const float*)params_flat, (const float*)z0, grid.d, B, T, ko,
                                  opts->norm_mode, (float*)traj_out, d_ret, d_na, d_nr, tape ? tape->t : nullptr,
                                  tape ? tape->dt : nullptr, tape ? (float*)tape->u : nullptr, tape ? tape->cap : 0, s);
     else if (dtype == LDEQ_F32)
-        rc = mlp_fwd_dispatch<float>(h, net, params_flat, z0, h->d_tgrid, B, T, ko, opts->norm_mode, traj_out, d_ret, d_na, d_nr, tape, s);
+        rc = mlp_fwd_dispatch<float>(h, net, params_flat, z0, grid.d, B, T, ko, opts->norm_mode, traj_out, d_ret, d_na, d_nr, tape, s);
     else
-        rc = mlp_fwd_dispatch<double>(h, net, params_flat, z0, h->d_tgrid, B, T, ko, opts->norm_mode, traj_out, d_ret, d_na, d_nr, tape, s);
+        rc = mlp_fwd_dispatch<double>(h, net, params_flat, z0, grid.d, B, T, ko, opts->norm_mode, traj_out, d_ret, d_na, d_nr, tape, s);
     if (rc) {
-        if (tape) { cudaFreeAsync(tape->base, s); cudaEventRecord(tape->ready, s); slot_release(h, tape->h_info, tape->ready); delete tape; }
+        if (tape) {
+            cudaFreeAsync(tape->base, s);
+            if (tape->ready) { cudaEventRecord(tape->ready, s); slot_release(h, tape->h_info, tape->ready); }
+            delete tape;
+        }
         return rc;
     }
     if (tape) {
-        // the reverse pass must know whether every accepted step found room on the tape (ldeq_mlp_solve_bwd checks)
+        // the reverse pass must know whether every accepted step found room on the tape (ldeq_mlp_solve_bwd checks it on
+        // the host for an eager tape, its gradient reduction on the device for a device-checked one)
         mlp_max_naccept_kernel<<<64, 256, 0, s>>>(tape->naccept, tape->retcode, B, tape->info);
         h->launches += 1;
-        cudaMemcpyAsync(tape->h_info, tape->info, 4, cudaMemcpyDeviceToHost, s);
-        cudaEventRecord(tape->ready, s);
+        if (tape->ready) {
+            cudaMemcpyAsync(tape->h_info, tape->info, 4, cudaMemcpyDeviceToHost, s);
+            cudaEventRecord(tape->ready, s);
+        }
         if (retcode) cudaMemcpyAsync(retcode, tape->retcode, (size_t)B * 4, cudaMemcpyDeviceToDevice, s);
         if (naccept) cudaMemcpyAsync(naccept, tape->naccept, (size_t)B * 4, cudaMemcpyDeviceToDevice, s);
         if (nreject) cudaMemcpyAsync(nreject, tape->nreject, (size_t)B * 4, cudaMemcpyDeviceToDevice, s);
         *tape_out = tape;
     }
     return LDEQ_OK;
+}
+
+extern "C" {
+
+int ldeq_mlp_solve_fwd(ldeq_handle* h, int dtype, const void* z0, const void* params_flat, const int32_t* layer_dims_host,
+                       int n_layers, const double* t_host, int B, int T, const ldeq_opts* opts, void* traj_out,
+                       int32_t* retcode, int32_t* naccept, int32_t* nreject, ldeq_mlp_tape** tape_out,
+                       ldeq_stream stream) {
+    if (!h) return LDEQ_ERR_INVALID;
+    if (tape_out) *tape_out = nullptr;
+    if (int rc0 = refuse_capture(h, (cudaStream_t)stream, "ldeq_mlp_solve_fwd", "its tape records the accepted-step count for a host-side check")) return rc0;
+    return mlp_solve_fwd(false, h, dtype, z0, params_flat, layer_dims_host, n_layers, t_host, B, T, opts, traj_out, retcode, naccept,
+                         nreject, nullptr, tape_out, (cudaStream_t)stream);
+}
+
+int ldeq_mlp_solve_fwd_dev(ldeq_handle* h, int dtype, const void* z0, const void* params_flat, const int32_t* layer_dims_host,
+                           int n_layers, const double* t_host, int B, int T, const ldeq_opts* opts, void* traj_out,
+                           int32_t* retcode, int32_t* naccept, int32_t* nreject, int32_t* overflow, ldeq_mlp_tape** tape_out,
+                           ldeq_stream stream) {
+    if (!h) return LDEQ_ERR_INVALID;
+    if (tape_out) *tape_out = nullptr;
+    return mlp_solve_fwd(true, h, dtype, z0, params_flat, layer_dims_host, n_layers, t_host, B, T, opts, traj_out, retcode, naccept,
+                         nreject, overflow, tape_out, (cudaStream_t)stream);
 }
 
 }  // extern "C"
@@ -597,7 +668,8 @@ static int launch_mlp_bwd(ldeq_handle* h, ldeq_mlp_tape* tape, const void* dtraj
                                                                      tape->naccept, (S*)dz0, (S*)h->scratch[1]);
     }
     LDEQ_CUDA(cudaGetLastError());
-    mlp_reduce_grads_kernel<S><<<(net.n_params + 255) / 256, 256, 0, s>>>((const S*)h->scratch[1], grid, net.n_params, (S*)dparams);
+    mlp_reduce_grads_kernel<S><<<(net.n_params + 255) / 256, 256, 0, s>>>((const S*)h->scratch[1], grid, net.n_params, (S*)dparams,
+                                                                          tape->info, tape->cap, tape->overflow);
     LDEQ_CUDA(cudaGetLastError());
     h->launches += 3;
     return LDEQ_OK;
@@ -694,16 +766,23 @@ int ldeq_mlp_solve_bwd(ldeq_handle* h, ldeq_mlp_tape* tape, const void* dtraj, v
     if (!h) return LDEQ_ERR_INVALID;
     if (!tape || !dtraj || !dz0 || !dparams_flat) return set_err(h, LDEQ_ERR_INVALID, "null argument");
     cudaStream_t s = (cudaStream_t)stream;
-    if (int rc0 = refuse_capture(h, s, "ldeq_mlp_solve_bwd", "it waits for the forward kernel to check the tape for overflow on the host")) return rc0;
+    // a device-checked tape (ldeq_mlp_solve_fwd_dev) never waits for the host: its gradient reduction applies the overflow
+    // rule on the device (mlp_tape_overflowed), and its tensor-core records are strided by the tape's capacity
+    const bool dev = tape->overflow != nullptr;
+    if (!dev) {
+        if (int rc0 = refuse_capture(h, s, "ldeq_mlp_solve_bwd", "it waits for the forward kernel to check the tape for overflow on the host")) return rc0;
+    }
     LDEQ_CUDA(cudaSetDevice(h->device));
-    // a solve that took more accepted steps than the tape holds has no exact gradient: say so instead of returning
-    // NaN / partial sums (waits for the forward kernel, as the GOKU path's tape check does)
-    LDEQ_CUDA(cudaEventSynchronize(tape->ready));
-    if (tape->h_info[0] > tape->cap) {
-        char msg[200];
-        snprintf(msg, sizeof msg, "mlp tape overflow: the solve accepted %d steps, the tape holds %d; repeat ldeq_mlp_solve_fwd "
-                 "with opts.tape_steps >= %d", tape->h_info[0], tape->cap, tape->h_info[0]);
-        return set_err(h, LDEQ_ERR_TAPE_OVERFLOW, msg);
+    if (!dev) {
+        // a solve that took more accepted steps than the tape holds has no exact gradient: say so instead of returning
+        // NaN / partial sums (waits for the forward kernel, as the GOKU path's tape check does)
+        LDEQ_CUDA(cudaEventSynchronize(tape->ready));
+        if (tape->h_info[0] > tape->cap) {
+            char msg[200];
+            snprintf(msg, sizeof msg, "mlp tape overflow: the solve accepted %d steps, the tape holds %d; repeat ldeq_mlp_solve_fwd "
+                     "with opts.tape_steps >= %d", tape->h_info[0], tape->cap, tape->h_info[0]);
+            return set_err(h, LDEQ_ERR_TAPE_OVERFLOW, msg);
+        }
     }
     if (tape->sense == LDEQ_SENSE_INTERPOLATING_ADJOINT) {
         if (tape->norm_mode != LDEQ_NORM_GLOBAL)
@@ -720,14 +799,14 @@ int ldeq_mlp_solve_bwd(ldeq_handle* h, ldeq_mlp_tape* tape, const void* dtraj, v
         for (int l = 0; l <= tape->net.n_layers; ++l) dims[l] = tape->net.dims[l];
         return ldeq_mlp_tc_backward(h, dims, tape->net.n_layers, (const float*)tape->params, tape->tgrid, tape->B, tape->T,
                                     (const float*)dtraj, tape->t, tape->dt, (float*)tape->u, tape->cap, tape->retcode, tape->naccept,
-                                    tape->h_info[0], (float*)dz0, (float*)dparams_flat, s);
+                                    dev ? tape->cap : tape->h_info[0], tape->info, tape->overflow, (float*)dz0, (float*)dparams_flat, s);
     }
     const bool small = tape->B <= 4 * h->sm_count;
     if (tape->dtype == LDEQ_F32 && !getenv("LDEQ_MLP_NO_RESIDENT")) {
         MlpTapeView<float> tv{tape->t, tape->dt, (float*)tape->u, tape->cap};
         const int rc = ldeq_mlp_res_backward(h, tape->net, (const float*)tape->params, tape->tgrid, tape->B, tape->T,
                                              (const float*)dtraj, tv, tape->retcode, tape->naccept, (float*)dz0,
-                                             (float*)dparams_flat, s);
+                                             (float*)dparams_flat, tape->info, tape->overflow, s);
         if (rc != LDEQ_ERR_UNSUPPORTED) return rc;
     }
     if (tape->dtype == LDEQ_F32)

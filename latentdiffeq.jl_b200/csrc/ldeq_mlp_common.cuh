@@ -651,10 +651,12 @@ static inline bool res_layout_ok(const MlpNet& net, int TB, int NT = RES_THREADS
 
 // ldeq_mlp_res.cu: Float32 weights resident in shared memory.  Both return LDEQ_ERR_UNSUPPORTED (without touching the
 // handle's error text) when the network / batch does not fit that path; the caller then uses the general kernels.
+// info / overflow: the tape's largest accepted-step count and, for a device-checked tape, its overflow word (null for an
+// eager tape), read by the gradient reduction (mlp_tape_overflowed).
 struct ldeq_mlp_tape;
 int ldeq_mlp_res_forward(ldeq_handle* h, const ldeq::MlpNet& net, const float* params, const float* z0, const double* d_tgrid,
                          int B, int T, const ldeq::KOpts& ko, int norm_mode, float* traj, int32_t* ret, int32_t* na, int32_t* nr,
                          ldeq::MlpTapeView<float> tv, double* partials, cudaStream_t s);
 int ldeq_mlp_res_backward(ldeq_handle* h, const ldeq::MlpNet& net, const float* params, const double* d_tgrid, int B, int T,
                           const float* dtraj, ldeq::MlpTapeView<float> tv, const int32_t* ret, const int32_t* na, float* dz0,
-                          float* dparams, cudaStream_t s);
+                          float* dparams, const int32_t* info, int32_t* overflow, cudaStream_t s);

@@ -327,8 +327,10 @@ template <int TB> static size_t bwd_res_smem(const MlpNet& net) {
 }
 
 template <class S> __global__ void mlp_res_reduce_grads_kernel(const S* __restrict__ gscratch, int n_cta, int n_params,
-                                                               S* __restrict__ dparams) {
+                                                               S* __restrict__ dparams, const int32_t* info, int cap, int32_t* overflow) {
+    const bool over = mlp_tape_overflowed(info, cap, overflow);
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_params; i += gridDim.x * blockDim.x) {
+        if (over) { dparams[i] = s_nan<S>(); continue; }
         double a = 0.0;
         for (int c = 0; c < n_cta; ++c) a += (double)gscratch[(size_t)c * n_params + i];
         dparams[i] = (S)a;
@@ -349,7 +351,7 @@ static int launch_res_fwd(ldeq_handle* h, const MlpNet& net, const float* P, con
     KOpts kov = ko;
     void* args[] = {&netv, &P, &z0, &tg, &B, &T, &kov, &traj, &ret, &na, &nr, &tv, &partials};
     if (GLOBAL) {
-        LDEQ_CUDA(cudaLaunchCooperativeKernel((void*)kern, dim3(grid), dim3(NT), args, smem, s));
+        LDEQ_CUDA(launch_cooperative((const void*)kern, dim3(grid), dim3(NT), args, smem, s));
     } else {
         LDEQ_CUDA(cudaLaunchKernel((void*)kern, dim3(grid), dim3(NT), args, smem, s));
     }
@@ -391,7 +393,7 @@ int ldeq_mlp_res_forward(ldeq_handle* h, const MlpNet& net, const float* P, cons
 
 int ldeq_mlp_res_backward(ldeq_handle* h, const MlpNet& net, const float* P, const double* tg, int B, int T, const float* dtraj,
                           MlpTapeView<float> tv, const int32_t* ret, const int32_t* na, float* dz0, float* dparams,
-                          cudaStream_t s) {
+                          const int32_t* info, int32_t* overflow, cudaStream_t s) {
     constexpr int TB = 2;
     const size_t smem = bwd_res_smem<TB>(net);
     if (!res_layout_ok(net, TB) || smem > kSmemMax) return LDEQ_ERR_UNSUPPORTED;
@@ -405,7 +407,8 @@ int ldeq_mlp_res_backward(ldeq_handle* h, const MlpNet& net, const float* P, con
     res_plan(netv, RES_THREADS);
     mlp_bwd_res_kernel<TB><<<grid, RES_THREADS, smem, s>>>(netv, P, tg, B, T, dtraj, tv, ret, na, dz0, (float*)h->scratch[1]);
     LDEQ_CUDA(cudaGetLastError());
-    mlp_res_reduce_grads_kernel<float><<<(net.n_params + 255) / 256, 256, 0, s>>>((const float*)h->scratch[1], grid, net.n_params, dparams);
+    mlp_res_reduce_grads_kernel<float><<<(net.n_params + 255) / 256, 256, 0, s>>>((const float*)h->scratch[1], grid, net.n_params, dparams,
+                                                                                 info, tv.cap, overflow);
     LDEQ_CUDA(cudaGetLastError());
     h->launches += 2;
     return LDEQ_OK;

@@ -454,7 +454,7 @@ int ldeq_mlp_tc_forward(ldeq_handle* h, const int32_t* dims, int n_layers, const
         if (tiles > h->sm_count)
             return set_err(h, LDEQ_ERR_UNSUPPORTED, "bf16x3 tensor-core path, global norm: B <= 128 * SM count (all tiles co-resident)");
         LDEQ_CUDA(cudaFuncSetAttribute(mlp_tc_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, net.smem_bytes));
-        LDEQ_CUDA(cudaLaunchCooperativeKernel((void*)mlp_tc_fwd_kernel<true>, dim3(tiles), dim3(TC_THREADS), args, net.smem_bytes, s));
+        LDEQ_CUDA(launch_cooperative((const void*)mlp_tc_fwd_kernel<true>, dim3(tiles), dim3(TC_THREADS), args, net.smem_bytes, s));
     } else {
         const int grid = tiles < h->sm_count ? tiles : h->sm_count;
         LDEQ_CUDA(cudaFuncSetAttribute(mlp_tc_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, net.smem_bytes));

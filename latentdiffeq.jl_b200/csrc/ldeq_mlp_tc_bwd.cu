@@ -415,10 +415,13 @@ mlp_tc_adj_kernel(TcNet net, const unsigned char* __restrict__ img_global, const
             }
         }
         if (live) {
+            // failed trajectories get a zero gradient, tape overflow NaN (only a device-checked tape gets here with one)
             const bool ok = retcode[b] == RET_SUCCESS;
+            const bool over = ok && naccept[b] > tape.cap;
 #pragma unroll
             for (int i = 0; i < 8; ++i)
-                if (c0 + i < D) dz0[(size_t)b * D + c0 + i] = ok ? ubn[i] + dtraj[(size_t)b * D + c0 + i] : 0.f;
+                if (c0 + i < D)
+                    dz0[(size_t)b * D + c0 + i] = over ? __int_as_float(0x7fc00000) : ok ? ubn[i] + dtraj[(size_t)b * D + c0 + i] : 0.f;
         }
         __syncthreads();
     }
@@ -588,8 +591,10 @@ mlp_tc_wgrad_kernel(TcNet net, TcRec rec, const unsigned char* __restrict__ reco
 }
 
 // partials [grid][P2 | P1 | P3] -> dparams in Flux.destructure order (per layer vec(W) column-major with W (out, in), then b)
+// NaN everywhere when a device-checked tape overflowed (mlp_tape_overflowed)
 __global__ void mlp_tc_wgrad_reduce_kernel(TcNet net, int D, int H1, int H2, const float* __restrict__ partials, int nparts,
-                                           float* __restrict__ dparams) {
+                                           float* __restrict__ dparams, const int32_t* info, int cap, int32_t* overflow) {
+    const bool over = mlp_tape_overflowed(info, cap, overflow);
     const size_t stride = (size_t)net.n2 * net.n1 + (size_t)net.n1 * TC_G_FEATS + (size_t)net.n2 * TC_D_FEATS;
     const int o1 = 0, ob1 = H1 * D, o2 = ob1 + H1, ob2 = o2 + H2 * H1, o3 = ob2 + H2, ob3 = o3 + D * H2, total = ob3 + D;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
@@ -600,6 +605,7 @@ __global__ void mlp_tc_wgrad_reduce_kernel(TcNet net, int D, int H1, int H2, con
         else if (i < o3) { const int n = i - ob2; src = (size_t)n * net.n1 + H1; }                                                                // db2[n]: h1's constant-1 column
         else if (i < ob3) { const int k = (i - o3) / D, d = (i - o3) % D; src = (size_t)net.n2 * net.n1 + (size_t)net.n1 * TC_G_FEATS + (size_t)k * TC_D_FEATS + d; }  // dW3[d, k]
         else { const int d = i - ob3; src = (size_t)net.n2 * net.n1 + (size_t)net.n1 * TC_G_FEATS + (size_t)H2 * TC_D_FEATS + d; }                // db3[d]: h2's constant-1 row
+        if (over) { dparams[i] = __int_as_float(0x7fc00000); continue; }
         float s = 0.f;
         for (int p = 0; p < nparts; ++p) s += partials[(size_t)p * stride + src];
         dparams[i] = s;
@@ -610,16 +616,8 @@ __global__ void mlp_tc_wgrad_reduce_kernel(TcNet net, int D, int H1, int H2, con
 
 using namespace ldeq;
 
-// Host side: called from ldeq_mlp_solve_bwd for a tape recorded with LDEQ_MLP_MATH_BF16X3.  `max_na` = largest accepted-step
-// count of a successful trajectory (known to the caller from the forward pass).
-int ldeq_mlp_tc_backward(ldeq_handle* h, const int32_t* dims, int n_layers, const float* params, const double* d_tgrid, int B, int T,
-                         const float* dtraj, double* tape_t, double* tape_dt, float* tape_u, int tape_cap, const int32_t* ret,
-                         const int32_t* na, int max_na, float* dz0, float* dparams, cudaStream_t s) {
-    TcNet net;
-    int rc = ldeq_tc_make_net(h, dims, n_layers, &net);
-    if (rc) return rc;
-    const int D = dims[0], H1 = dims[1], H2 = dims[2];
-    const int tiles = (B + TC_ROWS - 1) / TC_ROWS;
+// The record layout of the reverse pass: one block per (tile, step, stage), `nsteps` step slots per tile.
+static TcRec tc_rec(const TcNet& net, int nsteps) {
     TcRec rec;
     rec.nch1 = net.n1 / 8; rec.nch2 = net.n2 / 8;
     {
@@ -630,10 +628,40 @@ int ldeq_mlp_tc_backward(ldeq_handle* h, const int32_t* dims, int n_layers, cons
         rec.slice_bytes = o;
     }
     rec.block_bytes = (TC_ROWS / TC_SLICE_ROWS) * rec.slice_bytes;
-    rec.nsteps = max_na > 0 ? max_na : 1;
+    rec.nsteps = nsteps > 0 ? nsteps : 1;
+    return rec;
+}
+
+static size_t tc_rec_bytes(const TcRec& rec, int tiles) { return (size_t)tiles * rec.nsteps * 7 * rec.block_bytes; }
+
+// Scratch slot 1 of ldeq_mlp_tc_backward with `nsteps` step slots per tile: the records (tiles x nsteps x 7 blocks) and the
+// tiles' step counts.
+int ldeq_mlp_tc_record_scratch(ldeq_handle* h, const int32_t* dims, int n_layers, int B, int nsteps, size_t* bytes) {
+    TcNet net;
+    int rc = ldeq_tc_make_net(h, dims, n_layers, &net);
+    if (rc) return rc;
+    const int tiles = (B + TC_ROWS - 1) / TC_ROWS;
+    *bytes = tc_rec_bytes(tc_rec(net, nsteps), tiles) + (size_t)tiles * sizeof(int) + 256;
+    return LDEQ_OK;
+}
+
+// Host side: called from ldeq_mlp_solve_bwd for a tape recorded with LDEQ_MLP_MATH_BF16X3.  `nsteps`: the record slots per
+// tile, at least the largest accepted-step count of a successful trajectory that fits the tape -- that count for an eager tape
+// (the caller has it from the host check), the tape's capacity for a device-checked one.  The kernels walk the records by the
+// step counts they find on the device (tile_nsteps), so only the stride between tiles depends on it.  info / cap / overflow:
+// the gradient reduction's overflow rule (mlp_tape_overflowed).
+int ldeq_mlp_tc_backward(ldeq_handle* h, const int32_t* dims, int n_layers, const float* params, const double* d_tgrid, int B, int T,
+                         const float* dtraj, double* tape_t, double* tape_dt, float* tape_u, int tape_cap, const int32_t* ret,
+                         const int32_t* na, int nsteps, const int32_t* info, int32_t* overflow, float* dz0, float* dparams, cudaStream_t s) {
+    TcNet net;
+    int rc = ldeq_tc_make_net(h, dims, n_layers, &net);
+    if (rc) return rc;
+    const int D = dims[0], H1 = dims[1], H2 = dims[2];
+    const int tiles = (B + TC_ROWS - 1) / TC_ROWS;
+    const TcRec rec = tc_rec(net, nsteps);
     const size_t wg_smem = (size_t)WG_STAGES * rec.slice_bytes + 1024;
     if (wg_smem > 227 * 1024) return set_err(h, LDEQ_ERR_UNSUPPORTED, "bf16x3 tensor-core reverse pass: record tiles do not fit in shared memory");
-    const size_t rec_bytes = (size_t)tiles * rec.nsteps * 7 * rec.block_bytes;
+    const size_t rec_bytes = tc_rec_bytes(rec, tiles);
     const int wg_grid = h->sm_count;
     const size_t part_floats = (size_t)net.n2 * net.n1 + (size_t)net.n1 * TC_G_FEATS + (size_t)net.n2 * TC_D_FEATS;
     // scratch: [2] weight images, [1] records + tile step counts, [3] per-CTA partial gradients
@@ -655,7 +683,7 @@ int ldeq_mlp_tc_backward(ldeq_handle* h, const int32_t* dims, int n_layers, cons
     mlp_tc_wgrad_kernel<<<wg_grid, WG_THREADS, wg_smem, s>>>(net, rec, records, tile_nsteps, tiles, partials);
     LDEQ_CUDA(cudaGetLastError());
     const int total = H1 * D + H1 + H2 * H1 + H2 + D * H2 + D;
-    mlp_tc_wgrad_reduce_kernel<<<(total + 255) / 256, 256, 0, s>>>(net, D, H1, H2, partials, wg_grid, dparams);
+    mlp_tc_wgrad_reduce_kernel<<<(total + 255) / 256, 256, 0, s>>>(net, D, H1, H2, partials, wg_grid, dparams, info, tape_cap, overflow);
     LDEQ_CUDA(cudaGetLastError());
     h->launches += 4;
     return LDEQ_OK;

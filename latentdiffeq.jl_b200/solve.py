@@ -9,6 +9,7 @@ PyTorch is plumbing here (device memory, streams, autograd glue); all arithmetic
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 from typing import Sequence
 
@@ -262,11 +263,14 @@ def debug_trig(x: torch.Tensor, which: int = 0):
 
 # ---- LatentODE path: one solve on the (D,B) matrix state with an MLP right-hand side ---------------
 def mlp_solve_raw(z0: torch.Tensor, params_flat: torch.Tensor, dims: Sequence[int], t, opts: _cabi.Opts | None = None,
-                  want_tape: bool = False):
+                  want_tape: bool = False, overflow: torch.Tensor | None = None):
     """One call of ``ldeq_mlp_solve_fwd`` (reference ``src/models/LatentODE.jl:61-78``).
 
     ``z0`` is ``[B, D]``; ``params_flat`` is ``Flux.destructure`` order; ``dims = [D, H1, ..., D]``.
-    Returns ``(traj[T,B,D], stats, tape_or_None)``."""
+    Returns ``(traj[T,B,D], stats, tape_or_None)``.  ``overflow`` (a one-element int32 CUDA tensor): ``ldeq_mlp_solve_fwd_dev``
+    instead -- the same results, capture-safe, and a tape whose pullback never waits for the host: when the solve accepted
+    more steps N than the tape holds, ``mlp_bwd_raw`` returns NaN gradients and raises ``overflow`` to N (sticky) instead
+    of raising ``LdeqError``."""
     if not z0.is_cuda:
         raise RuntimeError("mlp_solve_raw needs CUDA tensors (there is no CPU implementation of the hot path)")
     h = _cabi.handle(z0.device.index or 0)
@@ -284,10 +288,15 @@ def mlp_solve_raw(z0: torch.Tensor, params_flat: torch.Tensor, dims: Sequence[in
     nr = torch.empty(B, dtype=torch.int32, device=z0.device)
     tape = C.c_void_p()
     with torch.cuda.device(z0.device):
-        h.check(h._lib.ldeq_mlp_solve_fwd(h.ptr, _dtype_code(z0.dtype), _p(z0), _p(params_flat),
-                                          dims_a.ctypes.data_as(C.c_void_p), len(dims_a) - 1,
-                                          tg.ctypes.data_as(C.c_void_p), B, T, C.byref(opts), _p(traj), _p(ret), _p(na),
-                                          _p(nr), C.byref(tape) if want_tape else None, _stream()))
+        args = (h.ptr, _dtype_code(z0.dtype), _p(z0), _p(params_flat), dims_a.ctypes.data_as(C.c_void_p), len(dims_a) - 1,
+                tg.ctypes.data_as(C.c_void_p), B, T, C.byref(opts), _p(traj), _p(ret), _p(na), _p(nr))
+        tape_arg = C.byref(tape) if want_tape else None
+        if overflow is not None:
+            if not (overflow.is_cuda and overflow.dtype == torch.int32 and overflow.numel() == 1):
+                raise TypeError("mlp_solve_raw: overflow must be one int32 element on the CUDA device")
+            h.check(h._lib.ldeq_mlp_solve_fwd_dev(*args, _p(overflow), tape_arg, _stream()))
+        else:
+            h.check(h._lib.ldeq_mlp_solve_fwd(*args, tape_arg, _stream()))
     tp = None
     if want_tape:
         tp = _Tape(h, tape, mlp=True)
@@ -316,11 +325,28 @@ def mlp_bwd_stats(tape: _Tape):
     return int(out[0]), int(out[1]), int(out[2])
 
 
+_tape_check = None
+
+
+@contextlib.contextmanager
+def device_tape_check(flag: torch.Tensor):
+    """Inside the block ``mlp_solve`` records device-checked tapes (``ldeq_mlp_solve_fwd_dev``) with the overflow word
+    ``flag`` (one int32 element on the CUDA device): the LatentODE solve and its pullback are then capture-safe.  A pullback
+    whose tape was too short gives NaN gradients and raises ``flag`` to the accepted-step count it needed, instead of
+    raising ``LdeqError``; only the caller clears ``flag``.  Outside the block nothing changes."""
+    global _tape_check
+    prev, _tape_check = _tape_check, flag
+    try:
+        yield
+    finally:
+        _tape_check = prev
+
+
 class _MlpSolve(torch.autograd.Function):
     @staticmethod
     def forward(ctx, z0, params_flat, tg, dims, opts, stats_out):
         need = z0.requires_grad or params_flat.requires_grad
-        traj, stats, tape = mlp_solve_raw(z0, params_flat, dims, tg, opts, want_tape=need)
+        traj, stats, tape = mlp_solve_raw(z0, params_flat, dims, tg, opts, want_tape=need, overflow=_tape_check)
         ctx.tape = tape
         if stats_out is not None:
             stats_out.append(stats)

@@ -13,7 +13,7 @@ import torch.distributed as dist
 
 from . import _cabi
 from . import model as _model
-from .solve import _tgrid, adamw_state, adamw_step, adamw_step_dev, allreduce_adamw_step, elbo_loss
+from .solve import _tgrid, adamw_state, adamw_step, adamw_step_dev, allreduce_adamw_step, device_tape_check, elbo_loss
 
 
 def loss_batch(model, x, t, beta, variational, fused_output: bool = True, unit_cotangent: bool = False, grad_scale: float = 1.0):
@@ -168,13 +168,24 @@ class GraphedTrainStep:
     calls in between (a validation ``loss_batch``) keep working on the same handle and stream; when the mirrors moved
     without the graph (an eager ``train_step``), the device state is refreshed from them before the replay.
 
-    Built for single-GPU GOKU training on its default path: Pendulum / Pendulum_friction / NVRTC right-hand sides with
-    ``ForwardDiffSensitivity()``, the pattern-extractor kernels, the fused logits ELBO and AdamW.  Everything else is refused
-    before any capture: LatentODE (its reverse passes need the host), ``DiscreteAdjoint()``, world size > 1 and a
-    reconstructor without the sigmoid output layer the fused loss needs.  ``x`` must keep ``x_example``'s shape, ``t`` is
-    fixed, and the noise seed is ``torch.initial_seed()`` at construction.  Construction warms the exact shapes up on a side
-    stream (modules, the device grid, the workspaces) and leaves parameters, gradients, ``m``, ``v``, ``opt.step_count`` and
-    the sample counter as it found them."""
+    Built for single-GPU training with the pattern-extractor kernels, the fused logits ELBO and AdamW, of
+    - GOKU on its default path: Pendulum / Pendulum_friction / NVRTC right-hand sides with ``ForwardDiffSensitivity()``;
+    - LatentODE when the NODE's sensitivity algorithm is ``DiscreteAdjoint()`` -- given explicitly, or the default with the
+      per-trajectory norm (``norm_mode=1``) or the bf16x3 tensor cores (``mlp_math=1``).  Its solve records device-checked
+      tapes (``device_tape_check``).
+    Everything else is refused before any capture: GOKU with ``DiscreteAdjoint()``, LatentODE with ``InterpolatingAdjoint()``
+    (the continuous adjoint sizes its buffers from a host count), world size > 1 and a reconstructor without the sigmoid
+    output layer the fused loss needs.  ``x`` must keep ``x_example``'s shape, ``t`` is fixed, and the noise seed is
+    ``torch.initial_seed()`` at construction.  Construction warms the exact shapes up on a side stream (modules, the device
+    grid, the workspaces) and leaves parameters, gradients, ``m``, ``v``, ``opt.step_count`` and the sample counter as it
+    found them.
+
+    Tape overflow (LatentODE with adaptive steps): a solve that accepts more steps than its tape holds (``tape_steps`` of the
+    NODE's kwargs, by default ``max(4 T, 256)``) cannot be differentiated exactly.  An eager step raises ``LdeqError``; a
+    replay cannot, so it follows the reference's own convention for failed solves (NaN, SURVEY.md Appendix C.8): that step's
+    gradient is NaN, AdamW writes NaN parameters, and ``tape_overflow()`` reports the step count the tape needed.  Check
+    ``tape_overflow()`` whenever the loss is read, and on a non-zero value rebuild the model's NODE with
+    ``NODE(..., tape_steps=n)`` for some n at or above it."""
 
     def __init__(self, model, flat: FlatParams, opt: ADAMW, x_example: torch.Tensor, t, variational: bool = True, warmup: int = 2):
         if not x_example.is_cuda:
@@ -183,13 +194,18 @@ class GraphedTrainStep:
             raise NotImplementedError("GraphedTrainStep: single GPU only (the gradient all-reduce is not captured)")
         if flat.symm is not None:
             raise NotImplementedError("GraphedTrainStep: FlatParams(symmetric=True) belongs to the fused multi-GPU step")
-        if not isinstance(model.model_type, _model.GOKU):
-            raise NotImplementedError("GraphedTrainStep: GOKU models only; LatentODE's reverse passes need the host (the MLP tape "
-                                      "check and the continuous adjoint)")
         diffeq = model.decoder.diffeq
         opts = _model._opts_from_kwargs(diffeq.kwargs, getattr(diffeq, "sensealg", None), getattr(diffeq, "solver", None))
-        if opts.sensealg != _cabi.SENSE_FORWARD_DUAL:
-            raise NotImplementedError("GraphedTrainStep: ForwardDiffSensitivity() only; the discrete adjoint checks its tape on the host")
+        if isinstance(model.model_type, _model.GOKU):
+            if opts.sensealg != _cabi.SENSE_FORWARD_DUAL:
+                raise NotImplementedError("GraphedTrainStep: ForwardDiffSensitivity() only; the discrete adjoint checks its tape on the host")
+        elif isinstance(model.model_type, _model.LatentODE):
+            if opts.sensealg != _cabi.SENSE_DISCRETE_ADJOINT:
+                raise NotImplementedError("GraphedTrainStep: LatentODE with InterpolatingAdjoint() cannot be captured (the continuous "
+                                          "adjoint sizes its buffers from the accepted-step count on the host); use "
+                                          "NODE(..., sensealg=DiscreteAdjoint())")
+        else:
+            raise NotImplementedError("GraphedTrainStep: GOKU and LatentODE models only")
         if _model._logits_layers(model.decoder) is None:
             raise NotImplementedError("GraphedTrainStep: the reconstructor must end in a Dense layer with the sigmoid output "
                                       "activation (the fused logits ELBO)")
@@ -200,6 +216,7 @@ class GraphedTrainStep:
         self._beta = torch.zeros((), dtype=torch.float32, device=dev)
         self._state = torch.zeros(3, dtype=torch.float64, device=dev)   # ldeq_adamw_state
         self._calls = torch.zeros(1, dtype=torch.int64, device=dev)
+        self._overflow = torch.zeros(1, dtype=torch.int32, device=dev)   # device-checked MLP tapes (device_tape_check)
         saved = [b.clone() for b in (flat.flat, flat.grad, flat.m, flat.v)]
         step0, calls0 = opt.step_count, _model._sample_calls
         cur = torch.cuda.current_stream(dev)
@@ -211,6 +228,7 @@ class GraphedTrainStep:
         cur.wait_stream(side)
         for b, v in zip((flat.flat, flat.grad, flat.m, flat.v), saved):
             b.copy_(v)
+        self._overflow.zero_()   # tape_overflow() speaks of replays only
         opt.step_count = step0
         _model._sample_calls = calls0
         self._graph = torch.cuda.CUDAGraph()
@@ -222,7 +240,7 @@ class GraphedTrainStep:
 
     def _body(self):
         self.flat.zero_grad()
-        with _model.device_sample_counter(self._calls):
+        with _model.device_sample_counter(self._calls), device_tape_check(self._overflow):
             loss = loss_batch(self.model, self._x, self._t, self._beta, self.variational, unit_cotangent=True)
         loss.backward()
         self.opt.step_dev(self._state)
@@ -244,3 +262,8 @@ class GraphedTrainStep:
         _model._sample_calls += self._draws
         self._synced = (self.opt.step_count, _model._sample_calls)
         return self._loss.clone()
+
+    def tape_overflow(self) -> int:
+        """0 when every replay so far found room on its LatentODE tapes; else the largest accepted-step count a tape would
+        have needed (the ``tape_steps`` to rebuild the NODE with).  Sticky across replays; synchronises the device."""
+        return int(self._overflow.item())

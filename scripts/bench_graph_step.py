@@ -1,10 +1,15 @@
 """Eager ``train_step`` against ``GraphedTrainStep`` on one GPU.
 
-    python scripts/bench_graph_step.py [--batches 64,8192] [--steps 500] [--block 25] [--warmup 20] [--out DIR]
+    python scripts/bench_graph_step.py [--model goku|latentode] [--batches ...] [--steps 500] [--block 25] [--warmup 20] [--out DIR]
 
-Workloads: the default GOKU-net (``default_layers``, Pendulum, adaptive Tsit5, ForwardDiffSensitivity, fused logits ELBO,
-AdamW) on 784-pixel ``bench.synthetic_frames`` of T = 50 frames, at the reference's batch of 64 (BASELINE.md C1) and at
-8192 as a no-regression check.  Both modes train the same model in one process, alternating blocks of ``--block`` steps
+Workloads, on 784-pixel ``bench.synthetic_frames`` of T = 50 frames:
+- ``goku`` (default): the default GOKU-net (``default_layers``, Pendulum, adaptive Tsit5, ForwardDiffSensitivity, fused
+  logits ELBO, AdamW) at the reference's batch of 64 (BASELINE.md C1) and at 8192 as a no-regression check;
+  writes ``graph_step.json``.
+- ``latentode``: ``default_layers(LatentODE(), 784, NODE(16, sensealg=DiscreteAdjoint()))`` (adaptive Tsit5 with the
+  batch-global norm on the resident-weights kernels, fused logits ELBO, AdamW) at the reference's batch of 64 and at 256
+  (BASELINE.md C2); writes ``graph_step_latentode.json``.
+Both modes train the same model in one process, alternating blocks of ``--block`` steps
 until each has run ``--steps``; every block is timed with CUDA events (the step time of a block is its time over its
 steps).  Writes ``graph_step.json`` under ``--out`` with the median and spread of the step time and samples/s per mode, the
 libldeq kernel launches of one eager step, and the GPU's name and power limit read in the same run."""
@@ -41,7 +46,16 @@ def stats(ms_per_step, batch):
             "samples_per_s_p10": float(np.percentile(sps, 10)), "samples_per_s_p90": float(np.percentile(sps, 90)), "blocks": len(a)}
 
 
-def run(batch, steps, block, warmup, dev):
+def build_model(kind, dev):
+    if kind == "goku":
+        mt, diffeq = ldeq.GOKU_basic(), ldeq.Pendulum()
+    else:
+        mt, diffeq = ldeq.LatentODE(), ldeq.NODE(16, sensealg=ldeq.DiscreteAdjoint())
+    enc, dec = ldeq.default_layers(mt, P_IN, diffeq, device=dev)
+    return ldeq.LatentDiffEqModel(mt, enc, dec)
+
+
+def run(kind, batch, steps, block, warmup, dev):
     torch.manual_seed(333)
     z0, th = pendulum_inputs(batch + 64, seed=1)
     with torch.no_grad():
@@ -55,8 +69,7 @@ def run(batch, steps, block, warmup, dev):
         return frames[o:o + T, b:b + batch]
 
     xs = [batch_at(k).contiguous() for k in range(8)]
-    enc, dec = ldeq.default_layers(ldeq.GOKU_basic(), P_IN, ldeq.Pendulum(), device=dev)
-    model = ldeq.LatentDiffEqModel(ldeq.GOKU_basic(), enc, dec)
+    model = build_model(kind, dev)
     flat = ldeq.FlatParams(model)
     opt = ldeq.ADAMW(flat, 1e-3, (0.9, 0.999), 1e-3)
     graphed = ldeq.GraphedTrainStep(model, flat, opt, xs[0], t)
@@ -83,6 +96,8 @@ def run(batch, steps, block, warmup, dev):
             times[mode].append(e0.elapsed_time(e1) / block)
         done += block
     assert torch.isfinite(loss).all()
+    if kind == "latentode":
+        assert graphed.tape_overflow() == 0
     out = {"batch": batch, "T": T, "pixels": P_IN, "steps_per_mode": done, "block": block,
            "eager": stats(times["eager"], batch), "graph": stats(times["graph"], batch), "libldeq_launches_per_eager_step": launches}
     out["speedup_median"] = out["eager"]["step_ms_median"] / out["graph"]["step_ms_median"]
@@ -91,7 +106,8 @@ def run(batch, steps, block, warmup, dev):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--batches", default="64,8192")
+    ap.add_argument("--model", choices=("goku", "latentode"), default="goku")
+    ap.add_argument("--batches", default=None, help="default: 64,8192 for goku, 64,256 for latentode")
     ap.add_argument("--steps", type=int, default=500)
     ap.add_argument("--block", type=int, default=25)
     ap.add_argument("--warmup", type=int, default=20)
@@ -100,9 +116,12 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench_graph_step.py measures on a CUDA device; there is none")
     dev = torch.device("cuda", 0)
-    res = {"gpu": gpu_info(), "workloads": [run(int(b), args.steps, args.block, args.warmup, dev) for b in args.batches.split(",")]}
+    batches = args.batches or ("64,8192" if args.model == "goku" else "64,256")
+    res = {"gpu": gpu_info(), "workloads": [run(args.model, int(b), args.steps, args.block, args.warmup, dev) for b in batches.split(",")]}
+    if args.model == "latentode":
+        res["model"] = "latentode"
     os.makedirs(args.out, exist_ok=True)
-    with open(os.path.join(args.out, "graph_step.json"), "w") as f:
+    with open(os.path.join(args.out, "graph_step.json" if args.model == "goku" else "graph_step_latentode.json"), "w") as f:
         json.dump(res, f, indent=1)
     print(json.dumps({"gpu": res["gpu"], "workloads": [{k: w[k] for k in ("batch", "speedup_median")} | {
         "eager_ms": w["eager"]["step_ms_median"], "graph_ms": w["graph"]["step_ms_median"]} for w in res["workloads"]]}))
